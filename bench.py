@@ -16,6 +16,7 @@ One step = sensor.encrypt() + knet.forward() over one batch.
   python bench.py --net lenet|acn|vgg16 [--batch B] [--parallel dp|rows|rows-fused]      (one workload only)
   python bench.py --mode keycompile                 (BASELINE configs[4]: key-compile sweep over the VGG16 layers)
   python bench.py --impl reference ...              (CPU arm: the oracle port of the reference's scipy path, all host threads)
+  python bench.py ... --dump-outputs DIR            (also write the logits of the last timed step of every workload as DIR/<net>_logits.npy)
 
 `value` = whole-job images/s with inputs resident in HBM; `e2e` = the same through the host-buffer API (pinned H2D of
 the images and D2H of the logits inside the timed region); `roofline` = the dominant launch against the measured peaks
@@ -43,6 +44,7 @@ HBM_FALLBACK_GBS = 6650.0     # /opt/skills/guides/B200_PROFILING.md fallback wh
 VGG_BATCH = 256
 LENET_BATCH = 65536
 ACN_BATCH = 4096
+DUMP_BYTES = 64 * 10**6       # --dump-outputs: at most this much in all
 
 
 # =================================================================================================
@@ -551,9 +553,10 @@ def _reduce_max(vals, world):
     return [float(v) for v in t]
 
 
-def bench_replicas(name, batch, K, warmup, rank, world, local_rank, want_cpu=True, cpu_budget_s=15.0, scaling='weak'):
+def bench_replicas(name, batch, K, warmup, rank, world, local_rank, want_cpu=True, cpu_budget_s=15.0, scaling='weak', outputs=None):
     """One GPU holds the whole keyed network; N > 1 = data-parallel replicas, no collective on the data path.
-    `batch` = images per GPU per step.  Returns the record on rank 0 (None elsewhere)."""
+    `batch` = images per GPU per step.  Returns the record on rank 0 (None elsewhere); `outputs` (a dict) receives the
+    logits of the last timed step as '<name>_logits'."""
     import torch
     from keynet_b200 import system, engine
     wl = workload(name)
@@ -585,6 +588,8 @@ def bench_replicas(name, batch, K, warmup, rank, world, local_rank, want_cpu=Tru
     e1.record()
     _barrier(world)
     ms = e0.elapsed_time(e1)
+    if outputs is not None:
+        outputs[name + '_logits'] = plan.logits.cpu().numpy()
     launches = plan.launches_per_run * K
     per_layer = plan.layer_times_ms_mean(K)
     plan.time_layers = False
@@ -689,9 +694,10 @@ def bench_replicas(name, batch, K, warmup, rank, world, local_rank, want_cpu=Tru
     return rec
 
 
-def bench_rows(name, batch, K, warmup, rank, world, local_rank, fused=True, want_cpu=True):
+def bench_rows(name, batch, K, warmup, rank, world, local_rank, fused=True, want_cpu=True, outputs=None):
     """Strong scaling: ONE batch, every keyed layer's rows cut into `world` shards (keynet_b200/dist.py), activations
-    all-gathered per layer over NVLink (NCCL, or fused into the SpMM epilogue: NVLink peer stores)."""
+    all-gathered per layer over NVLink (NCCL, or fused into the SpMM epilogue: NVLink peer stores).  `outputs` (a dict)
+    receives the logits of the last timed step as '<name>_logits'."""
     import torch
     import torch.distributed as dist
     from keynet_b200 import dist as kdist
@@ -736,6 +742,8 @@ def bench_rows(name, batch, K, warmup, rank, world, local_rank, fused=True, want
     _barrier(world)
     ms = e0.elapsed_time(e1)
     y = y.clone()
+    if outputs is not None:
+        outputs[name + '_logits'] = y[:, :-1].cpu().numpy()      # drop the homogeneous coordinate, as forward() does
     # ---- end to end: pinned host batch in, logits out, on every rank (the batch is replicated: every rank encrypts it)
     host_in = [torch.randn((N,) + wl['inshape']).pin_memory() for _ in range(2)]
     Kout = int(y.shape[1]) - 1
@@ -890,6 +898,19 @@ def bench_keycompile(args, rank, local_rank):
 
 
 # =================================================================================================
+def dump_outputs(outdir, outputs):
+    """Write each array of `outputs` ({name: [rows, cols]}) as outdir/<name>.npy in float32, within DUMP_BYTES in all.  An array
+    larger than its share keeps a fixed, seeded sample of its rows (in order), the same rows on every run."""
+    os.makedirs(outdir, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(outputs)) - 4096           # room for the .npy header
+    for (name, a) in sorted(outputs.items()):
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.nbytes > share:
+            keep = max(1, share // (a.shape[1] * a.itemsize))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(outdir, name + '.npy'), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -903,7 +924,13 @@ def main():
     ap.add_argument('--no-extra', action='store_true', help='skip the lenet / acn sub-records of the default run')
     ap.add_argument('--parallel', default=None, choices=['dp', 'rows', 'rows-fused'],
                     help='N > 1: dp = replicas; rows = every keyed layer row-sharded + NCCL all-gather; rows-fused = SpMM epilogue stores to NVLink peers (default for vgg16)')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='write the logits of the last timed step of every workload as DIR/<net>_logits.npy (float32; rank 0; a seeded row sample beyond 64 MB in all)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.mode != 'forward'):
+        ap.error('--dump-outputs applies to the GPU forward benchmark only')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
 
     rank = int(os.environ.get('RANK', '0'))
@@ -932,20 +959,21 @@ def main():
     want_cpu = (world == 1) and not args.no_cpu_baseline
     default_batch = {'vgg16': VGG_BATCH, 'lenet': LENET_BATCH, 'acn': ACN_BATCH}
     K = args.steps
+    outputs = {} if (args.dump_outputs and rank == 0) else None
 
     if parallel == 'dp':
         b = args.batch or default_batch[head]
         if head == 'acn' and args.batch is None:
             b = max(128, ACN_BATCH // world)                  # SURVEY cfg 2: 4096 images in total, split over the GPUs
-        rec = bench_replicas(head, b, K, args.warmup, rank, world, local_rank, want_cpu=want_cpu, scaling='strong' if head in ('acn', 'vgg16') else 'weak')
+        rec = bench_replicas(head, b, K, args.warmup, rank, world, local_rank, want_cpu=want_cpu, scaling='strong' if head in ('acn', 'vgg16') else 'weak', outputs=outputs)
     else:
-        rec = bench_rows(head, args.batch or default_batch[head], K, args.warmup, rank, world, local_rank, fused=(parallel == 'rows-fused'), want_cpu=want_cpu)
+        rec = bench_rows(head, args.batch or default_batch[head], K, args.warmup, rank, world, local_rank, fused=(parallel == 'rows-fused'), want_cpu=want_cpu, outputs=outputs)
     if args.net is None and not args.no_extra:
         torch.cuda.empty_cache()
         extra = {}
         for (nm, b, sc) in (('lenet', LENET_BATCH, 'weak'), ('acn', max(128, ACN_BATCH // world), 'strong')):
             try:
-                r = bench_replicas(nm, b, max(K, 10), args.warmup, rank, world, local_rank, want_cpu=want_cpu, cpu_budget_s=6.0, scaling=sc)
+                r = bench_replicas(nm, b, K, args.warmup, rank, world, local_rank, want_cpu=want_cpu, cpu_budget_s=6.0, scaling=sc, outputs=outputs)
             except Exception as e:             # a failing sub-record must not take the headline line with it (all ranks fail alike)
                 r = {'error': '%s: %s' % (type(e).__name__, str(e)[:300])}
             torch.cuda.empty_cache()
@@ -953,6 +981,8 @@ def main():
                 extra[nm] = r
         if rank == 0:
             rec['extra'] = extra
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0:
         print(json.dumps(rec))
     if dist.is_initialized():
