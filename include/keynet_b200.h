@@ -143,15 +143,20 @@ int kn_spmm_cg_f32(const int32_t *cl_gptr, const int32_t *cl_uptr, const int32_t
                    const int32_t *group_k, const int32_t *block_of, int64_t n_clusters, int32_t G, int32_t K_pad, int32_t u_max, int32_t g_max,
                    const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, uint32_t flags, const kn_peers *peers, void *stream);
 
-/* Tensor-core variant (csrc/pgroup_tc.cu): tcgen05.mma kind::tf32 with the 3xTF32 split (hi.hi + lo.hi + hi.lo),
- * fp32 accumulators in TMEM, weight blocks by TMA, gathered activations written into the UMMA layout by producer
- * warps.  kn_pg_tc_split: vals -> (hi = v & 0xffffe000, lo = v - hi); kn_pg_tc_tensormaps: writes four CUtensorMap
- * (4 x 128 bytes, HOST memory) describing the hi / lo planes [n_rows_total][K_pad] (full boxes, and half boxes for the
- * 2-CTA multicast launch); kn_spmm_pg_tc_f32: same contract
- * as kn_spmm_pg_f32 (results agree with fp32 FMA to ~1e-6 relative). */
+/* Tensor-core variant (csrc/pgroup_tc.cu): tcgen05.mma with an error-compensated split, per 8 k
+ *   x_hi.w_hi (kind::tf32)  +  [x_hi | x_lo] . [w_lo ; w_hi] (kind::f16 with bf16 operands, K = 16),
+ * both into one fp32 accumulator in TMEM (hi = v rounded to nearest TF32, lo = v - hi; error per product < 2^-16.9 |x||w|),
+ * weight blocks by TMA, gathered activations written into the UMMA layout by producer warps.
+ *   kn_pg_tc_split: vals[n] (n % 8 == 0, 16-byte aligned arrays) -> vals_hi[n]: hi as fp32 bit patterns, and vals_corr[n]:
+ *   per 8 consecutive values v[8j .. 8j+7], 8 words = 4 bf16 pairs of lo, then 4 bf16 pairs of hi (word i of each four
+ *   holds v[8j+2i] in its lower 16 bits and v[8j+2i+1] in its upper 16 bits).  Rows of length K_pad % 16 == 0 keep
+ *   every group of 8 inside a row.
+ *   kn_pg_tc_tensormaps: writes four CUtensorMap (4 x 128 bytes, HOST memory) describing the hi / corr planes
+ *   [n_rows_total][K_pad] of 4-byte words (full boxes, and half boxes for the 2-CTA multicast launch).
+ *   kn_spmm_pg_tc_f32: same contract as kn_spmm_pg_f32 (results agree with fp32 FMA to ~1e-6 relative). */
 #define KN_TENSORMAP_BYTES 128
-int kn_pg_tc_split(const float *vals, int64_t n, float *vals_hi, float *vals_lo, void *stream);
-int kn_pg_tc_tensormaps(const float *vals_hi, const float *vals_lo, int64_t n_rows_total, int32_t G, int32_t K_pad, void *maps_out_host);
+int kn_pg_tc_split(const float *vals, int64_t n, float *vals_hi, float *vals_corr, void *stream);
+int kn_pg_tc_tensormaps(const float *vals_hi, const float *vals_corr, int64_t n_rows_total, int32_t G, int32_t K_pad, void *maps_out_host);
 int kn_spmm_pg_tc_f32(const void *maps_host, const int32_t *rows, const int32_t *cols, const int32_t *group_k, const int32_t *block_of, int64_t n_groups, int32_t G, int32_t K_pad,
                       const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, uint32_t flags, const kn_peers *peers, void *stream);
 

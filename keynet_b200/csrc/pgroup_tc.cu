@@ -1,5 +1,5 @@
 // pgroup_tc.cu -- tensor-core kernel for the pattern-grouped format (kernel K4 of SURVEY.md 2.2):
-// tcgen05.mma kind::tf32 with the 3xTF32 error-compensated split, accumulators in TMEM.
+// tcgen05.mma with an error-compensated TF32 + BF16 split (2 MMAs per 8 k), fp32 accumulators in TMEM.
 //
 // Per pattern group g (see pgroup.cu) the product  Y[rows[g], :] = V_g (G x K) . X[cols[g], :] (K x N)
 // is a true small GEMM (G = 96..512 output channels, K = 9*Cin+1 = 865..4609, N = batch), which is what
@@ -9,17 +9,19 @@
 //
 //     D[128 batch][Gp] (TMEM, fp32)  +=  A[128 batch][8 k] (smem, MN-major)  .  B[8 k][Gp] (smem, K-major)
 //
-//   * B = weight block V_g: pre-split at pack time into hi = v & 0xffffe000 (exactly representable in
-//     TF32) and lo = v - hi, stored K-contiguous, loaded by TMA (SWIZZLE_64B boxes of 16 k x Gp rows).
+//   * B = weight block V_g: pre-split at pack time (kn_pg_tc_split) into a hi plane (v rounded to nearest TF32) and a
+//     corr plane of bf16 pairs ([w_lo ; w_hi] per 8 k, lo = v - hi), both K-contiguous 4-byte words, loaded by TMA
+//     (SWIZZLE_64B boxes of 16 words x Gp rows).
 //   * A = gathered activation rows X[cols[g][k], n0:n0+128], kept in TENSOR MEMORY (lane = batch element,
-//     column = k): eight producer warps read coalesced 128-byte row segments, split them into hi/lo in
-//     registers and write both with tcgen05.st into a TMEM ring; the MMA takes A from TMEM, so shared memory
+//     column = k): eight producer warps read coalesced 128-byte row segments, split them into TF32 hi words and bf16
+//     [x_hi | x_lo] pairs in registers and write both with tcgen05.st into a TMEM ring; the MMA takes A from TMEM, so shared memory
 //     carries only the weight ring.  (A first version staged A in shared memory, in the MN-major
 //     SWIZZLE_128B_BASE32B layout -- the only MN-major layout tcgen05 accepts for 32-bit operands; it was
 //     bound by the 128 B/clk shared-memory port: 7 KB of operands per 48-cycle N=96 MMA.)
-//   * one elected thread issues, per 8-k step, hi.hi + lo.hi + hi.lo (fp32 accumulate in TMEM): the
-//     dropped lo.lo term is below 2^-22 relative, so results stay inside the fp32 rtol 1e-4 parity bar,
-//     which plain TF32 (10-bit mantissa) would not.
+//   * one elected thread issues, per 8-k step, x_hi.w_hi (kind::tf32, K = 8) and [x_hi | x_lo].[w_lo ; w_hi]
+//     (kind::f16 in bf16, K = 16: both correction products in ONE instruction that reads as many operand bytes as a tf32
+//     K = 8 one and runs at twice its rate), both into the same fp32 accumulator.  Error per product < 2^-16.9 |x||w|
+//     (tc_common.cuh), inside the fp32 rtol 1e-4 parity bar, which plain TF32 (10-bit mantissa) would not be.
 //   * stages of 16 k, ring of kStages (full/empty mbarriers, tcgen05.commit frees a stage), epilogue:
 //     tcgen05.ld 32x32b.x16 -> ReLU -> Y[rows[g][j]][n] (32 lanes = 32 consecutive batch columns = 128 B).
 //
@@ -39,7 +41,8 @@ constexpr int kSuperTiles = 8;         // rasterisation super-tile: 8 x 128 = 10
 
 // Shared memory holds only the weight ring; the activation operand lives in TMEM:
 //   TMEM columns [0, NB*Gp)                      fp32 accumulators, one Gp-wide block per batch tile
-//   TMEM columns [a0 + (sa*NB + b)*32, +32)      A ring: 16 hi columns then 16 lo columns (lane = batch element, column = k)
+//   TMEM columns [a0 + (sa*NB + b)*32, +32)      A ring: 16 TF32 hi columns (column = k), then per 8 k 4 columns of bf16
+//                                                x_hi pairs and 4 of bf16 x_lo pairs (lane = batch element)
 // A tf32 UMMA with N = 96 needs 4 KB of A and 3 KB of B per 48 cycles; with A in shared memory that is 146 B/clk, above
 // the 128 B/clk shared-memory port, so the tensor pipe starves.  From TMEM the A operand costs no shared-memory
 // bandwidth and the producers' stores (tcgen05.st) bypass shared memory as well.
@@ -49,9 +52,9 @@ __device__ long long g_tc_timing[8];
 __device__ int g_tc_timing_cta = -1;
 #define KN_STAMP(i) do { if ((int)blockIdx.x == g_tc_timing_cta) g_tc_timing[i] = clock64(); } while (0)
 
-template <int NB, bool RELU, bool DUAL, int CS, bool PEERS>
+template <int NB, bool RELU, int CS, bool PEERS>
 __global__ void __launch_bounds__(kThreads, 1)
-pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo,
+pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_corr,
              const int32_t *__restrict__ rows, const int32_t *__restrict__ cols, const int32_t *__restrict__ group_k, const int32_t *__restrict__ block_of,
              int G, int Gp, int K_pad, int chunks_per_group, int64_t n_items, int64_t n_tiles, int n_b, int n_a, uint32_t a0, int super_tiles,
              const float *__restrict__ X, int64_t ldx, float *__restrict__ Y, int64_t ldy, int64_t n_vecs, const __grid_constant__ KnPeers peers)
@@ -59,7 +62,7 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
     extern __shared__ unsigned char smem_dyn[];
     unsigned char *smem = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~(uintptr_t)1023);
     const int b_plane_bytes = Gp * KS * 4;                       // Gp rows x 64 B
-    const int stage_bytes = 2 * b_plane_bytes;                   // hi plane, lo plane
+    const int stage_bytes = 2 * b_plane_bytes;                   // hi plane, corr plane
     int32_t *s_cols = reinterpret_cast<int32_t *>(smem + (size_t)n_b * stage_bytes);        // the group's gather list, K_pad entries
     uint64_t *fullB = reinterpret_cast<uint64_t *>(smem + (size_t)n_b * stage_bytes + (size_t)K_pad * 4);
     uint64_t *emptyB = fullB + n_b;
@@ -77,9 +80,6 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
     // groups of one class share K_pad (storage) but loop only over their own K (edge / corner pixels have fewer taps)
     const int n_ksteps = group_k ? (__ldg(group_k + g) + KS - 1) / KS : K_pad / KS;
     const uint32_t crank = (CS > 1) ? cluster_ctarank() : 0u;
-    // DUAL (Gp <= 128): the hi and lo weight planes are adjacent in shared memory, so ONE UMMA with N = 2*Gp computes
-    // x_hi.[w_hi ; w_lo] into two accumulator blocks (summed in the epilogue): 2 instructions per k-step instead of 3.
-    const int acc_w = DUAL ? 2 * Gp : Gp;                        // accumulator columns per batch tile
 
     if (tid == 0) KN_STAMP(0);
     if (warp == 0 && lane == 0) {
@@ -104,7 +104,7 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
     if (tid == 0) KN_STAMP(1);
 
     if (warp == 0) {
-        // ===== TMA producer: weight block planes (hi, lo), 16 k x Gp rows per stage =====
+        // ===== TMA producer: weight block planes (hi, corr), 16 k x Gp rows per stage =====
         if (elect_one()) {
             const int grow = (int)((block_of ? (int64_t)__ldg(block_of + g) : g) * G) + row0;      // rows of the group's unique value block
             int s = 0; uint32_t ph = 0;                          // ring position / phase kept incrementally (no runtime div/mod)
@@ -114,12 +114,12 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
                 mbar_arrive_expect_tx(&fullB[s], 2u * (uint32_t)b_plane_bytes);
                 if (CS == 1) {
                     tma_load_2d(bs, &map_hi, ks * KS, grow, &fullB[s]);
-                    tma_load_2d(bs + b_plane_bytes, &map_lo, ks * KS, grow, &fullB[s]);
+                    tma_load_2d(bs + b_plane_bytes, &map_corr, ks * KS, grow, &fullB[s]);
                 } else {
                     // this CTA fetches rows [rank*Gp/CS, (rank+1)*Gp/CS) of both planes and multicasts them to the cluster
                     const int part = Gp / CS, r0 = (int)crank * part;
                     tma_load_2d_mcast(bs + r0 * KS * 4, &map_hi, ks * KS, grow + r0, &fullB[s], (uint16_t)((1u << CS) - 1u));
-                    tma_load_2d_mcast(bs + b_plane_bytes + r0 * KS * 4, &map_lo, ks * KS, grow + r0, &fullB[s], (uint16_t)((1u << CS) - 1u));
+                    tma_load_2d_mcast(bs + b_plane_bytes + r0 * KS * 4, &map_corr, ks * KS, grow + r0, &fullB[s], (uint16_t)((1u << CS) - 1u));
                 }
                 if (++s == n_b) { s = 0; ph ^= 1u; }
             }
@@ -128,9 +128,9 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
         // ===== MMA issuers: one elected thread per batch tile (warp 1 -> batch tile 0, warp 3 -> batch tile 1) =====
         if (elect_one()) {
             const int b = (warp == 1) ? 0 : 1;
-            const uint32_t idesc = make_idesc(BM, Gp);
-            const uint32_t idesc2 = make_idesc(BM, 2 * Gp);
-            const uint32_t d = tmem_base + (uint32_t)(b * acc_w);
+            const uint32_t idesc = make_idesc_tf32(BM, Gp);
+            const uint32_t idesc_c = make_idesc_bf16(BM, Gp);
+            const uint32_t d = tmem_base + (uint32_t)(b * Gp);
             const uint64_t desc0 = make_desc(smem_u32(smem), 16, 512, kLayoutSW64);
             int sb = 0, sa = 0; uint32_t pb = 0, pa = 0;
             for (int ks = 0; ks < n_ksteps; ks++) {
@@ -140,20 +140,15 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
                 if (ks == 0 && warp == 1) KN_STAMP(2);
                 const uint32_t ta = tmem_base + a0 + (uint32_t)((sa * NB + b) * 32);
                 // B: K-major SW64 (64-byte rows), 8-row groups 512 B apart; stage / plane / k-step only move the
-                // 14-bit start-address field (units of 16 B), so the descriptor is one 64-bit add away from desc0
+                // 14-bit start-address field (units of 16 B), so the descriptor is one 64-bit add away from desc0.  An
+                // 8-k step is 32 B of a row in both planes: 8 tf32 words, or 16 bf16 (8 words) of the corr plane.
                 const uint64_t dstage = desc0 + (uint64_t)(((uint32_t)sb * (uint32_t)stage_bytes) >> 4);
 #pragma unroll
                 for (int kk = 0; kk < KS / 8; kk++) {
                     const uint64_t db_hi = dstage + (uint64_t)(kk * 2);
-                    const uint64_t db_lo = db_hi + (uint64_t)(b_plane_bytes >> 4);
-                    if (DUAL) {
-                        umma_tf32_ts(d, ta + kk * 8, db_hi, idesc2, (ks > 0 || kk > 0) ? 1u : 0u); // x_hi . [w_hi ; w_lo]
-                        umma_tf32_ts(d, ta + 16 + kk * 8, db_hi, idesc, 1u);                       // x_lo . w_hi
-                    } else {
-                        umma_tf32_ts(d, ta + kk * 8, db_hi, idesc, (ks > 0 || kk > 0) ? 1u : 0u);  // x_hi . w_hi
-                        umma_tf32_ts(d, ta + 16 + kk * 8, db_hi, idesc, 1u);                       // x_lo . w_hi
-                        umma_tf32_ts(d, ta + kk * 8, db_lo, idesc, 1u);                            // x_hi . w_lo
-                    }
+                    const uint64_t db_corr = db_hi + (uint64_t)(b_plane_bytes >> 4);
+                    umma_tf32_ts(d, ta + kk * 8, db_hi, idesc, (ks > 0 || kk > 0) ? 1u : 0u);    // x_hi . w_hi
+                    umma_bf16_ts(d, ta + 16 + kk * 8, db_corr, idesc_c, 1u);                     // x_hi . w_lo + x_lo . w_hi
                 }
                 if (CS == 1) umma_commit(&emptyB[sb]);         // both rings are released when every issuer's MMAs retire
                 else umma_commit_mcast(&emptyB[sb], (uint16_t)((1u << CS) - 1u));
@@ -165,7 +160,7 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
             if (warp == 1) KN_STAMP(3);
         }
     } else if (warp >= 4) {
-        // ===== A producers: gather X, split hi/lo, tcgen05.st into the TMEM A ring =====
+        // ===== A producers: gather X, split into TF32 hi + bf16 corr words, tcgen05.st into the TMEM A ring =====
         // thread = one batch element (TMEM lane); it loads X[cols[k]][n] for the k's of its stage share -- each warp
         // load is one coalesced 128-byte row segment -- and runs PD stages ahead of the TMEM stores (register ring).
         const int q = warp & 3;                                 // TMEM lane quarter of this warp
@@ -199,17 +194,14 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
         int psa = 0; uint32_t ppa = 0;                           // producer ring position / phase
         auto publish = [&](const float (&v)[KW]) {
             const int sa = psa;
-            uint32_t hi[KW], lo[KW];
+            uint32_t hi[KW], corr[KW];                          // corr: per 8 k, 4 bf16 x_hi pairs then 4 bf16 x_lo pairs
 #pragma unroll
-            for (int i = 0; i < KW; i++) {
-                hi[i] = __float_as_uint(v[i]) & 0xFFFFE000u;
-                lo[i] = __float_as_uint(v[i] - __uint_as_float(hi[i]));
-            }
+            for (int h = 0; h < KW / 8; h++) split8_tf32_bf16(v + 8 * h, hi + 8 * h, corr + 8 * h, corr + 8 * h + 4);
             mbar_wait(&emptyA[sa], ppa ^ 1u);
             tc_fence_after();
             const uint32_t ta = tmem_base + ((uint32_t)(q * 32) << 16) + a0 + (uint32_t)((sa * NB + b_mine) * 32 + k0);
             tmem_store<KW>(ta, hi);
-            tmem_store<KW>(ta + 16, lo);
+            tmem_store<KW>(ta + 16, corr);
         };
         // completing a stage (wait for the TMEM stores, then signal the issuers) is deferred until the next
         // gather has been issued, so the store latency overlaps with load issue instead of serialising every stage
@@ -245,18 +237,12 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
         for (int b = 0; b < NB; b++) {
             const int64_t ne = nbase + b * BM + q * 32 + lane;
             for (int c0 = half * 16; c0 < Gp; c0 += 32) {
-                uint32_t r[16], r2[16];
-                const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * acc_w + c0);
+                uint32_t r[16];
+                const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * Gp + c0);
                 asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
                              : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
                                "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
                              : "r"(taddr));
-                if (DUAL) {
-                    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                                 : "=r"(r2[0]), "=r"(r2[1]), "=r"(r2[2]), "=r"(r2[3]), "=r"(r2[4]), "=r"(r2[5]), "=r"(r2[6]), "=r"(r2[7]),
-                                   "=r"(r2[8]), "=r"(r2[9]), "=r"(r2[10]), "=r"(r2[11]), "=r"(r2[12]), "=r"(r2[13]), "=r"(r2[14]), "=r"(r2[15])
-                                 : "r"(taddr + (uint32_t)Gp));
-                }
                 asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
                 if (ne < n_vecs) {
                     if constexpr (!PEERS) {
@@ -264,7 +250,6 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
                         for (int t = 0; t < 16; t++) {
                             if (c0 + t < g_valid) {
                                 float y = __uint_as_float(r[t]);
-                                if (DUAL) y += __uint_as_float(r2[t]);
                                 if (RELU) y = fmaxf(y, 0.0f);
                                 Y[(int64_t)__ldg(rg + c0 + t) * ldy + ne] = y;
                             }
@@ -281,7 +266,6 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
 #pragma unroll
                         for (int t = 0; t < 16; t++) {
                             float y = __uint_as_float(r[t]);
-                            if (DUAL) y += __uint_as_float(r2[t]);
                             if (RELU) y = fmaxf(y, 0.0f);
                             r[t] = __float_as_uint(y);
                         }
@@ -308,14 +292,19 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
     }
 }
 
-// hi/lo split of a packed value array (weights): hi exactly representable in TF32
-__global__ void split_tf32_kernel(const float *__restrict__ v, int64_t n, float *__restrict__ hi, float *__restrict__ lo) {
+// split of a packed value array (weights), one thread per 8 consecutive k: hi = TF32 words, corr = 4 bf16 pairs of w_lo
+// then 4 of w_hi (the B operand of the kind::f16 correction MMA, against the A producers' [x_hi | x_lo])
+__global__ void split_tf32_kernel(const float *__restrict__ v, int64_t n8, uint32_t *__restrict__ hi, uint32_t *__restrict__ corr) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) {
-        const float x = v[i];
-        const float h = __uint_as_float(__float_as_uint(x) & 0xFFFFE000u);
-        hi[i] = h;
-        lo[i] = x - h;
+    if (i < n8) {
+        const float4 *src = reinterpret_cast<const float4 *>(v) + 2 * i;
+        const float4 a = src[0], b = src[1];
+        const float x[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+        uint32_t h[8], c[8];
+        split8_tf32_bf16(x, h, c + 4, c);
+        uint4 *dh = reinterpret_cast<uint4 *>(hi) + 2 * i, *dc = reinterpret_cast<uint4 *>(corr) + 2 * i;
+        dh[0] = make_uint4(h[0], h[1], h[2], h[3]); dh[1] = make_uint4(h[4], h[5], h[6], h[7]);
+        dc[0] = make_uint4(c[0], c[1], c[2], c[3]); dc[1] = make_uint4(c[4], c[5], c[6], c[7]);
     }
 }
 
@@ -341,7 +330,7 @@ static int tc_super_tiles() {
     return v > 0 ? v : kSuperTiles;
 }
 
-template <int NB, bool DUAL, int CS>
+template <int NB, int CS>
 int launch_tc(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols, const int32_t *group_k, const int32_t *block_of, int64_t n_groups, int G, int K_pad,
               const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, bool relu, cudaStream_t s)
 {
@@ -350,7 +339,7 @@ int launch_tc(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols,
     const int stage = 2 * Gp * KS * 4;
     int n_b = (int)((220 * 1024 - (int64_t)K_pad * 4) / stage);   // weight ring in shared memory, next to the column list
     if (n_b > 8) n_b = 8;
-    const uint32_t a0 = (uint32_t)(NB * (DUAL ? 2 * Gp : Gp));   // activation ring in TMEM, after the accumulators
+    const uint32_t a0 = (uint32_t)(NB * Gp);                     // activation ring in TMEM, after the accumulators
     int n_a = (int)((512 - a0) / (NB * 32));
     if (n_a > 6) n_a = 6;
     KN_REQUIRE(n_b >= 2 && n_a >= 2, "spmm_pg_tc: rings do not fit (Gp=%d NB=%d)", Gp, NB);
@@ -358,10 +347,10 @@ int launch_tc(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols,
     const int64_t gx = n_groups * chunks_per_group, gy = kn_cdiv(n_vecs, BM * NB);
     KN_REQUIRE(gx * gy <= 0x7fffffffLL, "spmm_pg_tc: grid too large");
     KN_ONCE_PER_DEVICE {
-        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, true, DUAL, CS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, false, DUAL, CS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, true, DUAL, CS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, false, DUAL, CS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, true, CS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, false, CS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, true, CS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, false, CS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     }
     const CUtensorMap *m = maps + (CS > 1 ? 2 : 0);              // maps[2..3]: boxes of Gp/2 rows for the multicast halves
     cudaLaunchConfig_t cfg = {};
@@ -377,7 +366,7 @@ int launch_tc(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols,
     const int n_b_ = n_b, n_a_ = n_a;
     const int super_ = tc_super_tiles() / NB > 0 ? tc_super_tiles() / NB : 1;
     const KnPeers peers = kn_current_peers();
-#define KN_TC_LAUNCH(R, P) KN_CUDA(cudaLaunchKernelEx(&cfg, pg_tc_kernel<NB, R, DUAL, CS, P>, m[0], m[1], rows, cols, group_k, block_of, G, Gp, K_pad, \
+#define KN_TC_LAUNCH(R, P) KN_CUDA(cudaLaunchKernelEx(&cfg, pg_tc_kernel<NB, R, CS, P>, m[0], m[1], rows, cols, group_k, block_of, G, Gp, K_pad, \
                                                      chunks_per_group, gx, gy, n_b_, n_a_, a0, super_, X, ldx, Y, ldy, n_vecs, peers))
     if (peers.n > 0) { if (relu) KN_TC_LAUNCH(true, true); else KN_TC_LAUNCH(false, true); }
     else             { if (relu) KN_TC_LAUNCH(true, false); else KN_TC_LAUNCH(false, false); }
@@ -386,7 +375,7 @@ int launch_tc(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols,
 }
 
 // cluster of 2 along the batch-tile axis whenever the tiles pair up inside a raster super-tile
-template <int NB, bool DUAL>
+template <int NB>
 int launch_tc_auto(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols, const int32_t *group_k, const int32_t *block_of, int64_t n_groups, int G, int K_pad,
                    const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, bool relu, cudaStream_t s)
 {
@@ -394,27 +383,29 @@ int launch_tc_auto(const CUtensorMap *maps, const int32_t *rows, const int32_t *
     const int64_t n_tiles = kn_cdiv(n_vecs, BM * NB);
     const int64_t S = tc_super_tiles() / NB > 0 ? tc_super_tiles() / NB : 1;
     const bool pairable = (n_tiles % 2 == 0) && (S % 2 == 0) && (Gp % 16 == 0) && ((n_tiles % S) % 2 == 0);
-    if (pairable) return launch_tc<NB, DUAL, 2>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s);
-    return launch_tc<NB, DUAL, 1>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s);
+    if (pairable) return launch_tc<NB, 2>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s);
+    return launch_tc<NB, 1>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s);
 }
 }  // namespace
 
-KN_API int kn_pg_tc_split(const float *vals, int64_t n, float *vals_hi, float *vals_lo, void *stream) {
-    KN_REQUIRE(n >= 0, "pg_tc_split: negative length");
+KN_API int kn_pg_tc_split(const float *vals, int64_t n, float *vals_hi, float *vals_corr, void *stream) {
+    KN_REQUIRE(n >= 0 && n % 8 == 0, "pg_tc_split: length must be a non-negative multiple of 8");
     if (n == 0) return KN_OK;
-    KN_REQUIRE(vals && vals_hi && vals_lo, "pg_tc_split: null pointer");
-    split_tf32_kernel<<<(unsigned)kn_cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>(vals, n, vals_hi, vals_lo);
+    KN_REQUIRE(vals && vals_hi && vals_corr, "pg_tc_split: null pointer");
+    KN_REQUIRE((((uintptr_t)vals | (uintptr_t)vals_hi | (uintptr_t)vals_corr) & 15) == 0, "pg_tc_split: arrays must be 16-byte aligned");
+    split_tf32_kernel<<<(unsigned)kn_cdiv(n / 8, 256), 256, 0, (cudaStream_t)stream>>>(vals, n / 8, reinterpret_cast<uint32_t *>(vals_hi),
+                                                                                     reinterpret_cast<uint32_t *>(vals_corr));
     KN_CHECK_LAUNCH();
     return KN_OK;
 }
 
-KN_API int kn_pg_tc_tensormaps(const float *vals_hi, const float *vals_lo, int64_t n_rows_total, int32_t G, int32_t K_pad, void *maps_out_host) {
-    KN_REQUIRE(vals_hi && vals_lo && maps_out_host, "pg_tc_tensormaps: null pointer");
+KN_API int kn_pg_tc_tensormaps(const float *vals_hi, const float *vals_corr, int64_t n_rows_total, int32_t G, int32_t K_pad, void *maps_out_host) {
+    KN_REQUIRE(vals_hi && vals_corr && maps_out_host, "pg_tc_tensormaps: null pointer");
     KN_REQUIRE(n_rows_total > 0 && G > 0 && K_pad > 0 && K_pad % KS == 0, "pg_tc_tensormaps: bad shape");
     PFN_encodeTiled enc = get_encode();
     if (!enc) { kn_set_error("cuTensorMapEncodeTiled is not available from this driver"); return KN_ERR_UNSUPPORTED; }
     const int Gp = (G > 256) ? 256 : ((G + 15) / 16) * 16;
-    const float *planes[4] = {vals_hi, vals_lo, vals_hi, vals_lo};
+    const float *planes[4] = {vals_hi, vals_corr, vals_hi, vals_corr};
     for (int i = 0; i < 4; i++) {
         CUtensorMap m;                                         // 64-byte aligned local; the caller's buffer need not be
         cuuint64_t dims[2] = {(cuuint64_t)K_pad, (cuuint64_t)n_rows_total};
@@ -445,14 +436,9 @@ KN_API int kn_spmm_pg_tc_f32(const void *maps_host, const int32_t *rows, const i
     const bool relu = (flags & KN_SPMM_RELU) != 0;
     const int Gp = (G > 256) ? 256 : ((G + 15) / 16) * 16;
     // two batch tiles per CTA share every weight stage when accumulators + a >= 2-deep activation ring fit TMEM
-    static const int use_dual = getenv("KN_TC_DUAL") ? atoi(getenv("KN_TC_DUAL")) : 1;   // experiment switch
-    if (use_dual && Gp <= 96 && n_vecs > BM)          // 2 tiles x 2*Gp accumulator columns + a 2-deep activation ring fit the 512 TMEM columns
-        return launch_tc_auto<2, true>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, (cudaStream_t)stream);
-    if (use_dual && Gp <= 128)
-        return launch_tc_auto<1, true>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, (cudaStream_t)stream);
     if (2 * Gp + 2 * 64 <= 512 && n_vecs > BM)
-        return launch_tc_auto<2, false>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, (cudaStream_t)stream);
-    return launch_tc_auto<1, false>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, (cudaStream_t)stream);
+        return launch_tc_auto<2>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, (cudaStream_t)stream);
+    return launch_tc_auto<1>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, (cudaStream_t)stream);
 }
 
 // debug: select the CTA whose phase timestamps are recorded (-1 = none) / read them back (7 x clock64)

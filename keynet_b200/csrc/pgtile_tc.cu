@@ -1,8 +1,9 @@
 // pgtile_tc.cu -- spatially tiled tensor-core kernel for keyed convolution layers with few output channels (G <= 128).
 //
 // pgroup_tc.cu runs one output pixel per CTA: for every 16-k stage it pulls 8 KB of gathered activations AND the pixel's
-// weight slab (hi + lo planes) from L2.  For G <= 128 that is ~64 B/clk/SM at full tensor rate, ~9.5 KB/clk over the chip,
-// against an L2 throughput cap of ~6.3 KB/clk: measured 49 % (G = 64) / 62 % (G = 128) of the 3xTF32 tensor ceiling, i.e.
+// weight slab (hi + corr planes) from L2.  For G <= 128 that is ~64 B/clk/SM at full tensor rate, ~9.5 KB/clk over the chip,
+// against an L2 throughput cap of ~6.3 KB/clk: measured 49 % (G = 64) / 62 % (G = 128) of the tensor ceiling of the former
+// 3xTF32 split (3 tf32 MMAs per 8 k), i.e.
 // those layers are bound by L2 -> SM traffic, not by the tensor pipe (VGG16 conv1_2 / conv2_x, AllConvNet conv2 / conv3).
 //
 // Here one CTA owns a TILE of th x tw neighbouring output pixels (2x2 for G <= 96, 1x2 for G <= 128) x 128 batch columns:
@@ -13,7 +14,7 @@
 //     (tap of pixel t at union position p = p - t*stride); taps that fall outside the image are simply not issued;
 //   * every pixel has its own fp32 accumulator in TMEM.  With stride 1 the pixels of one tile ROW that use a gathered position
 //     read CONSECUTIVE taps of one tap row (pixel tx at union column px uses tap dx = px - tx), so with the accumulators of a
-//     row laid out in descending tx and the hi (lo) planes of the tap slabs contiguous in shared memory, ONE tcgen05.mma of
+//     row laid out in descending tx and the hi (corr) planes of the tap slabs contiguous in shared memory, ONE tcgen05.mma of
 //     N = (pixels in the run) x Gp multiplies the stage by all of them (N = 128 .. 256 instead of 64 .. 128);
 //   * issuers are elected threads (kn_tc::elect_one -- under `if (lane == 0)` every tcgen05.mma cost 127-143 cycles of an
 //     ELECT / R2UR loop, under elect.sync one thread issues at the pipe rate), and an issuer is ONE thread running ~4-6 cycles
@@ -23,14 +24,16 @@
 //     geometries the whole schedule is folded at compile time (issuer_fast).  A slab is waited for once and released once
 //     per chunk and issuer (first / last use), not per use.  Other strides: one issuer and one instruction per (pixel, tap);
 //   * gathers: seven warps, cp.async 16 B per lane into a raw shared-memory ring that completes on mbarriers (16 stages =
-//     128 KB in flight towards the SM for G = 64); two splitter groups (hi / lo split -> tcgen05.st) on alternate stages;
+//     128 KB in flight towards the SM for G = 64); two splitter groups (hi / corr split -> tcgen05.st) on alternate stages;
 //   * output rows are transposed through the (by then idle) gather ring and leave as 512-byte cp.async.bulk rows;
-//   * A operand (gathered activations, hi/lo split in registers) in a TMEM ring exactly as in pgroup_tc.cu; 3xTF32
-//     (hi.hi + lo.hi + hi.lo), bias as one extra stage reading the homogeneous row.
+//   * A operand (gathered activations, split in registers) in a TMEM ring exactly as in pgroup_tc.cu, and the same split:
+//     per 8 k x_hi.w_hi (kind::tf32) + [x_hi | x_lo].[w_lo ; w_hi] (kind::f16 in bf16) into one fp32 accumulator
+//     (tc_common.cuh); bias as one extra stage reading the homogeneous row.
 // L2 -> SM bytes per (pixel, 16-channel chunk): G = 64: 108 KB -> 50 KB, G = 96: 126 -> 59, G = 128: 216 -> 120.
 //
 // Weight layout (built by the host): Wt[G][K_pad] TAP-major, k = tap * C + c, bias at k = n_taps * C, zero padded to a
-// multiple of 16; hi / lo TF32 planes + TMA descriptors with boxes of 16 k x Gp rows (kn_pg_tc_split / kn_pg_tc_tensormaps).
+// multiple of 16; hi (TF32) / corr (bf16 pairs) planes + TMA descriptors with boxes of 16 words x Gp rows (kn_pg_tc_split /
+// kn_pg_tc_tensormaps).
 // Tile tables (kn_conv2d_tiles_index): cols[tile][position][C] = activation row of every (position, channel) under the
 // layer's input key (-1 = position outside the image), rows[tile][pixel][G] = output row of every (pixel, channel).
 #include "tc_common.cuh"
@@ -95,7 +98,7 @@ __device__ __forceinline__ void issuer_fast(int n_chunks, int n_a, uint32_t tmem
                                             uint64_t *fullA, uint64_t *emptyA, uint64_t *fullB, uint64_t *emptyB, int &sa, uint32_t &pa)
 {
     constexpr int UW = TW + 2, UH = TH + 2;
-    constexpr uint64_t lo_off = (uint64_t)((9u * GP * 64u) >> 4);           // 9 slots (slot = tap) of hi planes, then the lo planes
+    constexpr uint64_t corr_off = (uint64_t)((9u * GP * 64u) >> 4);         // 9 slots (slot = tap) of hi planes, then the corr planes
     for (int cc = 0; cc < n_chunks; cc++) {
         const uint32_t pb = (uint32_t)(cc & 1);
 #pragma unroll
@@ -111,10 +114,8 @@ __device__ __forceinline__ void issuer_fast(int n_chunks, int n_a, uint32_t tmem
                 const uint32_t ta = a_base + (uint32_t)(sa * 32 + KK0 * 8);
                 const uint64_t db_hi = desc0 + (uint64_t)((((uint32_t)tap0 * GP * 64u) >> 4) + KK0 * 2);
                 constexpr uint32_t dummy = 0; (void)dummy;
-                const uint32_t idesc = make_idesc(BM, m * GP);
-                umma_tf32_ts(d, ta, db_hi, idesc, 1u);                      // x_hi . w_hi
-                umma_tf32_ts(d, ta + 16, db_hi, idesc, 1u);                 // x_lo . w_hi
-                umma_tf32_ts(d, ta, db_hi + lo_off, idesc, 1u);             // x_hi . w_lo
+                umma_tf32_ts(d, ta, db_hi, make_idesc_tf32(BM, m * GP), 1u);                 // x_hi . w_hi
+                umma_bf16_ts(d, ta + 16, db_hi + corr_off, make_idesc_bf16(BM, m * GP), 1u); // x_hi . w_lo + x_lo . w_hi
                 if (tx_hi == TW - 1) umma_commit(&emptyB[tap0]);            // last use of this slab by this issuer in this chunk
                 umma_commit(&emptyA[sa]);
             } else {
@@ -128,7 +129,7 @@ __device__ __forceinline__ void issuer_fast(int n_chunks, int n_a, uint32_t tmem
 
 template <bool RELU, bool PEERS, int TH, int TW, int GP>
 __global__ void __launch_bounds__(kThreads, 1)
-pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo,
+pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_corr,
                   const int32_t *__restrict__ tile_cols, const int32_t *__restrict__ tile_rows, int32_t bias_col,
                   const TileGeom geo, const __grid_constant__ TileJobs jobs_tab, int64_t n_sp_tiles, int64_t n_btiles, int super_tiles,
                   const float *__restrict__ X, int64_t ldx, float *__restrict__ Y, int64_t ldy, int64_t n_vecs, const __grid_constant__ KnPeers peers)
@@ -188,10 +189,10 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
                 const int cc = j / geo.n_taps, tap = j - cc * geo.n_taps;
                 const int k0 = (j == n_slabs - 1) ? geo.n_taps * C : tap * C + cc * KS;
                 mbar_wait(&emptyB[s], ph ^ 1u);
-                unsigned char *bs = smem + (size_t)s * geo.plane_bytes;             // hi planes of all slots, then lo planes: consecutive taps are contiguous
+                unsigned char *bs = smem + (size_t)s * geo.plane_bytes;             // hi planes of all slots, then corr planes: consecutive taps are contiguous
                 mbar_arrive_expect_tx(&fullB[s], (uint32_t)geo.slab_bytes);
                 tma_load_2d(bs, &map_hi, k0, 0, &fullB[s]);
-                tma_load_2d(bs + (size_t)geo.n_slots * geo.plane_bytes, &map_lo, k0, 0, &fullB[s]);
+                tma_load_2d(bs + (size_t)geo.n_slots * geo.plane_bytes, &map_corr, k0, 0, &fullB[s]);
                 if (++s == geo.n_slots) { s = 0; ph ^= 1u; }
             }
         }
@@ -200,18 +201,18 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
         const int w = warp - 1;
         if (w < geo.n_iss && elect_one()) {
             const uint64_t desc0 = make_desc(smem_u32(smem), 16, 512, kLayoutSW64);
-            const uint64_t lo_off = (uint64_t)(((uint32_t)geo.n_slots * (uint32_t)geo.plane_bytes) >> 4);
+            const uint64_t corr_off = (uint64_t)(((uint32_t)geo.n_slots * (uint32_t)geo.plane_bytes) >> 4);
             const int kk0 = w % geo.ksplit;                         // this issuer's 8-k steps of a stage: kk0, kk0 + ksplit, ...
             const uint32_t a_base = tmem_base + geo.a0;
             const int4 *jobs = jobs_tab.rec + w * kMaxPos;
             int sa = 0; uint32_t pa = 0;
             auto issue = [&](uint32_t d, uint64_t dslab, uint32_t idesc) {     // every accumulator was zeroed by the splitters: always accumulate
                 const uint32_t ta = a_base + (uint32_t)(sa * 32);
+                const uint32_t idesc_c = idesc_tf32_to_bf16(idesc);
                 for (int kk = kk0; kk < KS / 8; kk += geo.ksplit) {
                     const uint64_t db_hi = dslab + (uint64_t)(kk * 2);
                     umma_tf32_ts(d, ta + kk * 8, db_hi, idesc, 1u);                // x_hi . w_hi
-                    umma_tf32_ts(d, ta + 16 + kk * 8, db_hi, idesc, 1u);           // x_lo . w_hi
-                    umma_tf32_ts(d, ta + kk * 8, db_hi + lo_off, idesc, 1u);       // x_hi . w_lo
+                    umma_bf16_ts(d, ta + 16 + kk * 8, db_hi + corr_off, idesc_c, 1u);   // x_hi . w_lo + x_lo . w_hi
                 }
             };
             bool fast = false;
@@ -270,7 +271,7 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
                 mbar_wait(&fullA[sa], pa);
                 tc_fence_after();
                 const int n_acc = geo.merged ? geo.tw : 1;
-                for (int a = 0; a < n_acc; a++) issue(tmem_base + (uint32_t)(((w / geo.ksplit) * n_acc + a) * Gp), desc0, make_idesc(BM, Gp));
+                for (int a = 0; a < n_acc; a++) issue(tmem_base + (uint32_t)(((w / geo.ksplit) * n_acc + a) * Gp), desc0, make_idesc_tf32(BM, Gp));
                 umma_commit(&emptyB[0]);
                 umma_commit(&emptyA[sa]);
             }
@@ -332,7 +333,7 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
         }
         asm volatile("cp.async.wait_all;\n" ::: "memory");
     } else if (warp >= kProducerWarp0) {
-        // ===== splitters: raw stage -> hi / lo TF32 planes -> tcgen05.st into the TMEM ring =====
+        // ===== splitters: raw stage -> TF32 hi / bf16 corr words -> tcgen05.st into the TMEM ring =====
         // two groups of four warps (one warp per TMEM lane quarter) take alternate stages, so the fixed latencies of one
         // stage's chain (barrier wait, shared-memory reads, TMEM store + wait, arrive) overlap with the other group's stage
         const int q = warp & 3;                                 // TMEM lane quarter
@@ -350,14 +351,13 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
             sa += 2; if (sa >= geo.n_a) { sa -= geo.n_a; aph ^= 1u; }
             { PROF_T0(20); mbar_wait(&raw_full[slot], rph); if (tid == kProducerWarp0 * 32) PROF_ADD(20); }
             const float *src = src0 + (size_t)slot * (KS * BM);
-            uint32_t hi[KS], lo[KS];
+            uint32_t hi[KS], corr[KS];                          // corr: per 8 k, 4 bf16 x_hi pairs then 4 bf16 x_lo pairs
             { PROF_T0(21);
+            float v[KS];
 #pragma unroll
-            for (int j = 0; j < KS; j++) {
-                const float v = src[j * BM];
-                hi[j] = __float_as_uint(v) & 0xFFFFE000u;
-                lo[j] = __float_as_uint(v - __uint_as_float(hi[j]));
-            }
+            for (int j = 0; j < KS; j++) v[j] = src[j * BM];
+#pragma unroll
+            for (int h = 0; h < KS / 8; h++) split8_tf32_bf16(v + 8 * h, hi + 8 * h, corr + 8 * h, corr + 8 * h + 4);
             mbar_arrive(&raw_empty[slot]);                      // the values are in registers: the slot can be refilled
             if (tid == kProducerWarp0 * 32) PROF_ADD(21); }
             { PROF_T0(23); mbar_wait(&emptyA[sa], aph); if (tid == kProducerWarp0 * 32) PROF_ADD(23); }
@@ -365,7 +365,7 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
             PROF_T0(24);
             const uint32_t ta = tmem_base + ((uint32_t)(q * 32) << 16) + geo.a0 + (uint32_t)(sa * 32);
             tmem_store<KS>(ta, hi);
-            tmem_store<KS>(ta + 16, lo);
+            tmem_store<KS>(ta + 16, corr);
             asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
             tc_fence_before();
             mbar_arrive(&fullA[sa]);
@@ -648,7 +648,7 @@ KN_API int kn_spmm_tile_tc_f32(const void *maps_host, const int32_t *tile_cols, 
             rec.x = 2 | (rel << 2) | (tap0 << 8) | ((acc0 * g.Gp) << 16);
             rec.y = (int)(((1u << m) - 1u) << tap0);
             rec.z = (int)(((uint32_t)tap0 * (uint32_t)g.plane_bytes) >> 4);          // slab ring of exactly n_taps slots: slot = tap
-            rec.w = (int)make_idesc(BM, m * g.Gp);
+            rec.w = (int)make_idesc_tf32(BM, m * g.Gp);
         }
     }
     CUtensorMap maps[4];

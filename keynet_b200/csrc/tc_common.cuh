@@ -70,9 +70,16 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr, uint32_t lbo_b
 }
 constexpr uint32_t kLayoutSW64 = 4;      // (SWIZZLE_128B_BASE32B = 1 is the only MN-major layout for 32-bit operands; not used: A lives in TMEM)
 
-// instruction descriptor (cute::UMMA::InstrDescriptor): D=f32, A=B=tf32, A (TMEM) and B K-major
-__host__ __device__ constexpr uint32_t make_idesc(int M, int N) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | (0u << 15) | (0u << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+// instruction descriptors (cute::UMMA::InstrDescriptor): D=f32, A (TMEM) and B K-major.  The A / B format field is the only
+// difference between the two kinds: tf32 (2) under kind::tf32, bf16 (1) under kind::f16.
+__host__ __device__ constexpr uint32_t make_idesc_fmt(int M, int N, uint32_t ab_format) {
+    return (1u << 4) | (ab_format << 7) | (ab_format << 10) | (0u << 15) | (0u << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+__host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N) { return make_idesc_fmt(M, N, 2u); }
+__host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N) { return make_idesc_fmt(M, N, 1u); }
+// the kind::f16 (bf16) descriptor of the same shape as a kind::tf32 one
+__host__ __device__ constexpr uint32_t idesc_tf32_to_bf16(uint32_t idesc_tf32) {
+    return idesc_tf32 ^ (make_idesc_tf32(0, 0) ^ make_idesc_bf16(0, 0));
 }
 
 // A operand from tensor memory: D[tmem] (+)= A[tmem] . B[smem desc]
@@ -82,6 +89,48 @@ __device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, u
         "setp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
         :: "r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
+// the same with bf16 operands (K = 16 per instruction, two elements per 32-bit TMEM column / 4-byte word of B); it may
+// accumulate into an accumulator that kind::tf32 instructions also write: both keep D in fp32
+__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+        :: "r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
+
+// The split of the tensor-core kernels (2 MMAs per 8 k):  x.w ~= x_hi.w_hi  (kind::tf32, K = 8)
+//                                                                + [x_hi | x_lo] . [w_lo ; w_hi]  (kind::f16 in bf16, K = 16)
+// hi = v rounded to nearest TF32, lo = v - hi (exact in fp32, |lo| <= 2^-11 |v|).  The correction terms are ~2^-11 of the
+// product, so bf16's 8-bit significand leaves them ~2^-18 of it; bf16 has fp32's exponent range (no scaling, where fp16
+// would underflow on x_lo).  Per product the error is below 1.04 * 2^-17 |x||w|: two cross terms of <= 2^-11 |x||w| whose
+// operands are rounded to bf16 (2^-8 each), plus the dropped lo.lo (<= 2^-22).  The former 3xTF32 split was ~3 * 2^-20;
+// both are far inside the rtol 1e-4 parity bar (tests/test_split_numerics.py models them).
+__device__ __forceinline__ uint32_t tf32_rna(float v) {
+    uint32_t h;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(h) : "f"(v));
+    return h & 0xFFFFE000u;                 // the tf32 value as an fp32 bit pattern
+}
+__device__ __forceinline__ uint32_t bf16x2_rn(float k_even, float k_odd) {        // the lower half holds the lower k
+    uint32_t r;
+    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(k_odd), "f"(k_even));
+    return r;
+}
+// 8 consecutive k of one row: hi[8] = TF32 words, bhi[4] / blo[4] = bf16 pairs of hi / lo (k = 2j in the lower half of word j)
+__device__ __forceinline__ void split8_tf32_bf16(const float *v, uint32_t *hi, uint32_t *bhi, uint32_t *blo) {
+    float h[8], l[8];
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        hi[i] = tf32_rna(v[i]);
+        h[i] = __uint_as_float(hi[i]);
+        l[i] = v[i] - h[i];
+    }
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        bhi[j] = bf16x2_rn(h[2 * j], h[2 * j + 1]);
+        blo[j] = bf16x2_rn(l[2 * j], l[2 * j + 1]);
+    }
 }
 
 template <int NW>
