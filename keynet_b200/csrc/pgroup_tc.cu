@@ -28,16 +28,12 @@
 // One CTA per (group, 128*NB batch columns); NB = 2 batch tiles share every weight stage.
 #include "tc_common.cuh"
 #include <string.h>
-#include <stdlib.h>
 
 namespace {
 using namespace kn_tc;
 
 constexpr int kThreads = 384;          // warp 0: TMA(B)  warps 1,3: MMA issuers  warp 2: TMEM alloc  warps 4-11: A producers + epilogue
 constexpr int kProducerThreads = 256;
-constexpr int KS = 16;                 // k per stage
-constexpr int BM = 128;                // batch columns per UMMA (M)
-constexpr int kSuperTiles = 8;         // rasterisation super-tile: 8 x 128 = 1024 batch columns (sweep 4..32: 4/8 best by ~1 %)
 
 // Shared memory holds only the weight ring; the activation operand lives in TMEM:
 //   TMEM columns [0, NB*Gp)                      fp32 accumulators, one Gp-wide block per batch tile
@@ -91,8 +87,7 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
         mbar_init(accum_bar, NB);
         fence_barrier_init();
     } else if (warp == 2) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" :: "r"(smem_u32(tmem_slot)));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+        tmem_alloc512(tmem_slot);
     }
     // the column list is read once per CTA: a gather then never waits for an index load before it can issue
     for (int i = tid; i < n_ksteps * KS; i += kThreads) s_cols[i] = __ldg(cols + g * (int64_t)K_pad + i);
@@ -238,45 +233,9 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
             const int64_t ne = nbase + b * BM + q * 32 + lane;
             for (int c0 = half * 16; c0 < Gp; c0 += 32) {
                 uint32_t r[16];
-                const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * Gp + c0);
-                asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                             : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-                               "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                             : "r"(taddr));
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                if (ne < n_vecs) {
-                    if constexpr (!PEERS) {
-#pragma unroll
-                        for (int t = 0; t < 16; t++) {
-                            if (c0 + t < g_valid) {
-                                float y = __uint_as_float(r[t]);
-                                if (RELU) y = fmaxf(y, 0.0f);
-                                Y[(int64_t)__ldg(rg + c0 + t) * ldy + ne] = y;
-                            }
-                        }
-                    } else {
-                        // fused all-gather (separate instantiation: this code costs the plain epilogue ~10 %): row ids and
-                        // need masks first, then one pass of NVLink stores per peer
-                        int32_t yrow[16];
-                        unsigned pmask[16];
-#pragma unroll
-                        for (int t = 0; t < 16; t++) yrow[t] = (c0 + t < g_valid) ? __ldg(rg + c0 + t) : -1;
-#pragma unroll
-                        for (int t = 0; t < 16; t++) pmask[t] = (yrow[t] >= 0) ? kn_peer_mask(peers, yrow[t]) : 0u;
-#pragma unroll
-                        for (int t = 0; t < 16; t++) {
-                            float y = __uint_as_float(r[t]);
-                            if (RELU) y = fmaxf(y, 0.0f);
-                            r[t] = __float_as_uint(y);
-                        }
-                        for (int p = 0; p < peers.n; p++) {
-                            float *__restrict__ yb = peers.y[p];
-#pragma unroll
-                            for (int t = 0; t < 16; t++)
-                                if ((pmask[t] >> p) & 1u) yb[(int64_t)yrow[t] * ldy + ne] = __uint_as_float(r[t]);
-                        }
-                    }
-                }
+                tmem_load16(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * Gp + c0), r);
+                if (ne < n_vecs)
+                    store_rows16<RELU, PEERS>(r, g_valid - c0, [&](int t) { return __ldg(rg + c0 + t); }, Y, ldy, ne, peers);
             }
         }
     }
@@ -286,10 +245,7 @@ pg_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__
     __syncthreads();
     if (tid == 0) KN_STAMP(6);
     if (CS > 1) cluster_sync_all();                              // no CTA leaves while a partner may still signal its barriers
-    if (warp == 2) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" :: "r"(tmem_base));
-    }
+    if (warp == 2) tmem_dealloc512(tmem_base);
 }
 
 // split of a packed value array (weights), one thread per 8 consecutive k: hi = TF32 words, corr = 4 bf16 pairs of w_lo
@@ -323,19 +279,12 @@ PFN_encodeTiled get_encode() {
     return fn;
 }
 
-// batch columns (in 128-column tiles) per raster super-tile: small enough that the X rows shared by neighbouring groups
-// (3x3 windows re-read every row 9 times, one image row of groups apart) are still L2-resident when they are re-read
-static int tc_super_tiles() {
-    static const int v = getenv("KN_TC_SUPER") ? atoi(getenv("KN_TC_SUPER")) : kSuperTiles;
-    return v > 0 ? v : kSuperTiles;
-}
-
 template <int NB, int CS>
 int launch_tc(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols, const int32_t *group_k, const int32_t *block_of, int64_t n_groups, int G, int K_pad,
               const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, bool relu, cudaStream_t s)
 {
     const int chunks_per_group = (G + 255) / 256;
-    const int Gp = (G > 256) ? 256 : ((G + 15) / 16) * 16;
+    const int Gp = tc_gp(G);
     const int stage = 2 * Gp * KS * 4;
     int n_b = (int)((220 * 1024 - (int64_t)K_pad * 4) / stage);   // weight ring in shared memory, next to the column list
     if (n_b > 8) n_b = 8;
@@ -346,12 +295,6 @@ int launch_tc(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols,
     const size_t smem = (size_t)n_b * stage + (size_t)K_pad * 4 + 1024 + 512;
     const int64_t gx = n_groups * chunks_per_group, gy = kn_cdiv(n_vecs, BM * NB);
     KN_REQUIRE(gx * gy <= 0x7fffffffLL, "spmm_pg_tc: grid too large");
-    KN_ONCE_PER_DEVICE {
-        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, true, CS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, false, CS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, true, CS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        KN_CUDA(cudaFuncSetAttribute(pg_tc_kernel<NB, false, CS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    }
     const CUtensorMap *m = maps + (CS > 1 ? 2 : 0);              // maps[2..3]: boxes of Gp/2 rows for the multicast halves
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(gx * gy));
@@ -363,27 +306,24 @@ int launch_tc(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols,
     attr[0].val.clusterDim.x = CS; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    const int n_b_ = n_b, n_a_ = n_a;
-    const int super_ = tc_super_tiles() / NB > 0 ? tc_super_tiles() / NB : 1;
     const KnPeers peers = kn_current_peers();
-#define KN_TC_LAUNCH(R, P) KN_CUDA(cudaLaunchKernelEx(&cfg, pg_tc_kernel<NB, R, CS, P>, m[0], m[1], rows, cols, group_k, block_of, G, Gp, K_pad, \
-                                                     chunks_per_group, gx, gy, n_b_, n_a_, a0, super_, X, ldx, Y, ldy, n_vecs, peers))
-    if (peers.n > 0) { if (relu) KN_TC_LAUNCH(true, true); else KN_TC_LAUNCH(false, true); }
-    else             { if (relu) KN_TC_LAUNCH(true, false); else KN_TC_LAUNCH(false, false); }
-#undef KN_TC_LAUNCH
-    return KN_OK;
+    return dispatch_relu_peers(relu, peers.n > 0, [&](auto R, auto P) {
+        const auto kfn = pg_tc_kernel<NB, decltype(R)::value, CS, decltype(P)::value>;
+        KN_ONCE_PER_DEVICE { KN_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); }
+        KN_CUDA(cudaLaunchKernelEx(&cfg, kfn, m[0], m[1], rows, cols, group_k, block_of, G, Gp, K_pad, chunks_per_group, gx, gy, n_b, n_a, a0,
+                                   kSuperTiles / NB, X, ldx, Y, ldy, n_vecs, peers));
+        return KN_OK;
+    });
 }
 
-// cluster of 2 along the batch-tile axis whenever the tiles pair up inside a raster super-tile
+// cluster of 2 along the batch-tile axis whenever the tiles pair up inside a raster super-tile: an even number of batch
+// tiles does, as a super-tile holds an even number of them
+static_assert((kSuperTiles / 2) % 2 == 0, "kSuperTiles / NB must be even");
 template <int NB>
 int launch_tc_auto(const CUtensorMap *maps, const int32_t *rows, const int32_t *cols, const int32_t *group_k, const int32_t *block_of, int64_t n_groups, int G, int K_pad,
                    const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, bool relu, cudaStream_t s)
 {
-    const int Gp = (G > 256) ? 256 : ((G + 15) / 16) * 16;
-    const int64_t n_tiles = kn_cdiv(n_vecs, BM * NB);
-    const int64_t S = tc_super_tiles() / NB > 0 ? tc_super_tiles() / NB : 1;
-    const bool pairable = (n_tiles % 2 == 0) && (S % 2 == 0) && (Gp % 16 == 0) && ((n_tiles % S) % 2 == 0);
-    if (pairable) return launch_tc<NB, 2>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s);
+    if (kn_cdiv(n_vecs, BM * NB) % 2 == 0) return launch_tc<NB, 2>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s);
     return launch_tc<NB, 1>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s);
 }
 }  // namespace
@@ -404,7 +344,7 @@ KN_API int kn_pg_tc_tensormaps(const float *vals_hi, const float *vals_corr, int
     KN_REQUIRE(n_rows_total > 0 && G > 0 && K_pad > 0 && K_pad % KS == 0, "pg_tc_tensormaps: bad shape");
     PFN_encodeTiled enc = get_encode();
     if (!enc) { kn_set_error("cuTensorMapEncodeTiled is not available from this driver"); return KN_ERR_UNSUPPORTED; }
-    const int Gp = (G > 256) ? 256 : ((G + 15) / 16) * 16;
+    const int Gp = tc_gp(G);
     const float *planes[4] = {vals_hi, vals_corr, vals_hi, vals_corr};
     for (int i = 0; i < 4; i++) {
         CUtensorMap m;                                         // 64-byte aligned local; the caller's buffer need not be
@@ -434,9 +374,8 @@ KN_API int kn_spmm_pg_tc_f32(const void *maps_host, const int32_t *rows, const i
     CUtensorMap maps[4];
     memcpy(maps, maps_host, 4 * sizeof(CUtensorMap));
     const bool relu = (flags & KN_SPMM_RELU) != 0;
-    const int Gp = (G > 256) ? 256 : ((G + 15) / 16) * 16;
     // two batch tiles per CTA share every weight stage when accumulators + a >= 2-deep activation ring fit TMEM
-    if (2 * Gp + 2 * 64 <= 512 && n_vecs > BM)
+    if (2 * tc_gp(G) + 2 * 64 <= 512 && n_vecs > BM)
         return launch_tc_auto<2>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, (cudaStream_t)stream);
     return launch_tc_auto<1>(maps, rows, cols, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, (cudaStream_t)stream);
 }

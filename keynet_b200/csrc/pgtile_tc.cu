@@ -38,20 +38,14 @@
 // layer's input key (-1 = position outside the image), rows[tile][pixel][G] = output row of every (pixel, channel).
 #include "tc_common.cuh"
 #include <string.h>
-#include <stdlib.h>
 
 namespace {
 using namespace kn_tc;
 
-#ifndef KN_TILE_GATHER_WARPS
-#define KN_TILE_GATHER_WARPS 7
-#endif
-constexpr int kGatherWarps = KN_TILE_GATHER_WARPS;
+constexpr int kGatherWarps = 7;
 constexpr int kProducerWarp0 = 12;     // first splitter warp: a multiple of 4 (a warp reaches the TMEM lanes of its quarter, warp % 4)
 constexpr int kThreads = (kProducerWarp0 + 8) * 32;   // warp 0: TMA (weight slabs)  warps 1-4: MMA issuers  warps 5..: activation gathers (cp.async; warp 7 first allocates TMEM)  warps 12-19: hi/lo splitters + epilogue
 constexpr int kGroupThreads = 128;     // the 8 splitter warps work as two groups of 4 (one warp per TMEM lane quarter) on alternate stages
-constexpr int KS = 16;                 // k per stage = channels per chunk
-constexpr int BM = 128;                // batch columns per CTA (UMMA M)
 constexpr int kMaxT = 4;               // output pixels per tile (issuer warps 1-4)
 constexpr int kGatherWarp0 = 5;        // warps 5 .. 5 + kGatherWarps - 1: activation gathers (stages round-robin)
 static_assert(kGatherWarp0 + kGatherWarps <= kProducerWarp0, "gather warps overlap the splitters");
@@ -79,11 +73,10 @@ struct TileGeom {
     int bulk_epi, epi_pixels;          // epilogue through shared memory + bulk copies: pixels per pass (0 = per-lane stores)
     uint32_t a0;                       // first TMEM column of the activation ring (after the T accumulators)
     int slab_bytes, plane_bytes;
-    unsigned char pos_order[kMaxPos];  // union positions in issue order: consecutive positions feed DISJOINT sets of pixels (see launch code)
 };
 
-// What every issuer does at every position of the issue order -- geometry only, the same for every tile, so it is built on the
-// host and travels as a kernel parameter (constant bank: a uniform load in the issuers' loop):
+// What every issuer does at every union position (issued in raster order) -- geometry only, the same for every tile, so it is
+// built on the host and travels as a kernel parameter (constant bank: a uniform load in the issuers' loop):
 //   x: bit 1 this issuer has MMAs here | bit 2 last use of slab (x >> 8 & 255) in the chunk | first accumulator column << 16
 //   y: taps read (bit per slab)      z: B descriptor offset (slot = tap)      w: instruction descriptor
 struct TileJobs { int4 rec[kMaxT * kMaxPos]; };
@@ -163,8 +156,7 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
         mbar_init(accum_bar, geo.n_iss);
         fence_barrier_init();
     } else if (warp == 7) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" :: "r"(smem_u32(tmem_slot)));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+        tmem_alloc512(tmem_slot);
     }
     // the tile's gather table and output rows: ONE global round trip and one barrier before every role starts (the stage list and
     // the issuers' records used to be built here behind a second barrier: 7 k cycles of prologue with the tensor pipe idle)
@@ -175,8 +167,8 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    unsigned vmask = 0;                                       // bit o: the o-th position of the issue order lies inside the image
-    for (int o = 0; o < U_pos; o++) vmask |= (s_cols[geo.pos_order[o] * C] >= 0 ? 1u : 0u) << o;
+    unsigned vmask = 0;                                       // bit p: union position p lies inside the image
+    for (int p = 0; p < U_pos; p++) vmask |= (s_cols[p * C] >= 0 ? 1u : 0u) << p;
     const int n_stages = geo.n_chunks * __popc(vmask) + 1;    // in-image (chunk, position) stages + the bias stage
     if (tid == 0) PROF_SET(1);
     const int n_slabs = geo.n_chunks * geo.n_taps + 1;
@@ -289,21 +281,17 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
         const float *__restrict__ xcol = X + (col_ok ? ncol : 0);
         const int bytes = col_ok ? 16 : 0;                      // src-size 0 => 16 bytes of zeros
         const int mine = warp - kGatherWarp0;
-        int i = -1, cc = 0, o = -1;                              // stage counter and its (chunk, position of the issue order)
+        int i = -1, cc = 0, p = -1;                              // stage counter and its (chunk, union position)
         int slot = -1, turn = kGatherWarps - 1; uint32_t rph = 1u;   // the stage's ring slot / the parity its raw_empty is waited with / whose turn it is
         while (true) {
             // next in-image stage, chunk-major; after the last chunk the bias stage (ring position kept incrementally: a runtime
             // division per stage is ~150 cycles of a gather warp's ~460)
-            int p;
             ++i;
             if (++slot == geo.n_raw) { slot = 0; rph ^= 1u; }
             if (++turn == kGatherWarps) turn = 0;
             if (i == n_stages - 1) p = kBiasPos;
             else if (i >= n_stages) break;
-            else {
-                do { if (++o == U_pos) { o = 0; ++cc; } } while (!((vmask >> o) & 1u));
-                p = geo.pos_order[o];
-            }
+            else do { if (++p == U_pos) { p = 0; ++cc; } } while (!((vmask >> p) & 1u));
             if (turn != mine) continue;
             { PROF_T0(30); mbar_wait(&raw_empty[slot], rph); if (tid == kGatherWarp0 * 32) PROF_ADD(30); }
             PROF_T0(31);
@@ -379,6 +367,9 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
         if (tid == kProducerWarp0 * 32) PROF_SET(4);
         const int half = sel;                                    // two warps per lane quarter: even / odd 16-column chunks
         const int64_t ne = nbase + q * 32 + lane;
+        const uint32_t t_lanes = tmem_base + ((uint32_t)(q * 32) << 16);
+        // accumulator of pixel t: those of a tile row are in descending tx (merged runs)
+        auto acc_of = [&](int t) { return geo.merged ? (t / geo.tw) * geo.tw + (geo.tw - 1 - t % geo.tw) : t; };
         if (!PEERS && geo.bulk_epi) {
             // Output rows through shared memory and bulk copies.  With per-lane stores (below) a warp instruction writes one
             // 128-byte piece of a row and the SM's queue of outstanding stores, not bandwidth, set the pace: 128 KB per CTA took
@@ -393,16 +384,10 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
                 const int tn = (T - t0 < ppp) ? T - t0 : ppp;
                 asm volatile("bar.sync 1, 256;" ::: "memory");  // the ring is idle (both splitter groups done) / the previous pass has been read
                 for (int tl = 0; tl < tn; tl++) {
-                    const int t = t0 + tl;
-                    const int acc = geo.merged ? (t / geo.tw) * geo.tw + (geo.tw - 1 - t % geo.tw) : t;
+                    const int acc = acc_of(t0 + tl);
                     for (int c0 = half * 16; c0 < Gp; c0 += 32) {
                         uint32_t r[16];
-                        const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * Gp + c0);
-                        asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                                     : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-                                       "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                                     : "r"(taddr));
-                        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                        tmem_load16(t_lanes + (uint32_t)(acc * Gp + c0), r);
                         float *dst = stage + (size_t)(tl * geo.G + c0) * BM + q * 32 + lane;
 #pragma unroll
                         for (int j = 0; j < 16; j++) {
@@ -428,49 +413,12 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
         } else
         for (int t = 0; t < T; t++) {
             const int32_t *rg = s_rows + t * 256;
-            const int acc = geo.merged ? (t / geo.tw) * geo.tw + (geo.tw - 1 - t % geo.tw) : t;      // accumulators of a tile row are in descending tx (merged runs)
+            const int acc = acc_of(t);
             for (int c0 = half * 16; c0 < Gp; c0 += 32) {
                 uint32_t r[16];
-                const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * Gp + c0);
-                { PROF_T0(40);
-                asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                             : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-                               "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                             : "r"(taddr));
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                if (tid == kProducerWarp0 * 32) PROF_ADD(40); }
+                { PROF_T0(40); tmem_load16(t_lanes + (uint32_t)(acc * Gp + c0), r); if (tid == kProducerWarp0 * 32) PROF_ADD(40); }
                 PROF_T0(41);
-                if (ne < n_vecs) {
-                    if constexpr (!PEERS) {
-#pragma unroll
-                        for (int j = 0; j < 16; j++) {
-                            if (c0 + j < geo.G) {
-                                float y = __uint_as_float(r[j]);
-                                if (RELU) y = fmaxf(y, 0.0f);
-                                Y[(int64_t)rg[c0 + j] * ldy + ne] = y;
-                            }
-                        }
-                    } else {
-                        int32_t yrow[16];
-                        unsigned pmask[16];
-#pragma unroll
-                        for (int j = 0; j < 16; j++) yrow[j] = (c0 + j < geo.G) ? rg[c0 + j] : -1;
-#pragma unroll
-                        for (int j = 0; j < 16; j++) pmask[j] = (yrow[j] >= 0) ? kn_peer_mask(peers, yrow[j]) : 0u;
-#pragma unroll
-                        for (int j = 0; j < 16; j++) {
-                            float y = __uint_as_float(r[j]);
-                            if (RELU) y = fmaxf(y, 0.0f);
-                            r[j] = __float_as_uint(y);
-                        }
-                        for (int pp = 0; pp < peers.n; pp++) {
-                            float *__restrict__ yb = peers.y[pp];
-#pragma unroll
-                            for (int j = 0; j < 16; j++)
-                                if ((pmask[j] >> pp) & 1u) yb[(int64_t)yrow[j] * ldy + ne] = __uint_as_float(r[j]);
-                        }
-                    }
-                }
+                if (ne < n_vecs) store_rows16<RELU, PEERS>(r, geo.G - c0, [&](int j) { return rg[c0 + j]; }, Y, ldy, ne, peers);
                 if (tid == kProducerWarp0 * 32) PROF_ADD(41);
             }
         }
@@ -480,10 +428,7 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
     tc_fence_before();
     __syncthreads();
     if (tid == 0) PROF_SET(6);
-    if (warp == 7) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" :: "r"(tmem_base));
-    }
+    if (warp == 7) tmem_dealloc512(tmem_base);
 }
 
 // ---- tile tables from the layer geometry -------------------------------------------------------------------------------
@@ -517,11 +462,6 @@ conv_tiles_index_kernel(kn_conv2d_desc d, const int32_t *__restrict__ tile_origi
             tile_rows[tl * (int64_t)T * d.M + i] = row_of_src ? row_of_src[s] : (int32_t)s;
         }
     }
-}
-
-int tile_super_tiles() {
-    static const int v = getenv("KN_TILE_SUPER") ? atoi(getenv("KN_TILE_SUPER")) : 8;
-    return v > 0 ? v : 8;
 }
 }  // namespace
 
@@ -559,9 +499,9 @@ KN_API int kn_spmm_tile_tc_f32(const void *maps_host, const int32_t *tile_cols, 
     KN_REQUIRE(n_vecs % 4 == 0 && ldx % 4 == 0 && (((uintptr_t)X) & 15) == 0, "spmm_tile_tc: n_vecs and ldx must be multiples of 4, X 16-byte aligned");
     KN_REQUIRE(ldx * 4 < 0xffffffffLL, "spmm_tile_tc: leading dimension in bytes must fit 32 bits");
     TileGeom g;
-    g.C = C; g.G = G; g.Gp = ((G + 15) / 16) * 16; g.th = th; g.tw = tw; g.T = th * tw; g.stride = stride; g.P = P; g.Q = Q; g.n_taps = P * Q;
+    g.C = C; g.G = G; g.Gp = tc_gp(G); g.th = th; g.tw = tw; g.T = th * tw; g.stride = stride; g.P = P; g.Q = Q; g.n_taps = P * Q;
     g.uh = (th - 1) * stride + P; g.uw = (tw - 1) * stride + Q; g.U_pos = g.uh * g.uw; g.n_chunks = C / KS;
-    KN_REQUIRE(g.T <= kMaxT && g.U_pos <= kMaxPos && g.Gp <= 256, "spmm_tile_tc: tile too large (T=%d positions=%d)", g.T, g.U_pos);
+    KN_REQUIRE(g.T <= kMaxT && g.U_pos <= kMaxPos && G <= 256, "spmm_tile_tc: tile too large (T=%d positions=%d)", g.T, g.U_pos);
     g.merged = (stride == 1 && tw * g.Gp <= 256) ? 1 : 0;
     g.ksplit = (g.merged && 2 * th <= kMaxT) ? 2 : 1;
     g.n_iss = g.merged ? th * g.ksplit : g.T;
@@ -580,53 +520,19 @@ KN_API int kn_spmm_tile_tc_f32(const void *maps_host, const int32_t *tile_cols, 
     int n_raw = (int)((avail - (int64_t)n_slots * g.slab_bytes) / kRawStageBytes);
     if (n_raw > 16) n_raw = 16;
     KN_REQUIRE(n_raw >= 3, "spmm_tile_tc: the weight slabs of one channel chunk do not fit shared memory (Gp=%d taps=%d)", g.Gp, g.n_taps);
-    // issue order of the union positions: raster order (taps are then consumed in the order the slabs load), or -- experiment
-    // switch KN_TILE_ORDER=1 -- rounds of positions that feed pairwise DISJOINT pixel sets so that the issuers work on
-    // different stages at the same time (measured on B200: 7.30 vs 7.28 ms on VGG16 conv1_2, no gain).
-    {
-        unsigned mask_of[kMaxPos];
-        for (int p = 0; p < g.U_pos; p++) {
-            const int py = p / g.uw, px = p - py * g.uw;
-            unsigned m = 0;
-            for (int t = 0; t < g.T; t++) {
-                const int ty = t / g.tw, tx = t - ty * g.tw;
-                const int dy = py - ty * g.stride, dx = px - tx * g.stride;
-                if (dy >= 0 && dy < g.P && dx >= 0 && dx < g.Q) m |= 1u << t;
-            }
-            mask_of[p] = m;
-        }
-        bool done[kMaxPos] = {false};
-        int n_out = 0;
-        static const int balanced = getenv("KN_TILE_ORDER") ? atoi(getenv("KN_TILE_ORDER")) : 0;       // measured: no gain over raster order (the issuers are not the limiter); kept as a switch
-        while (n_out < g.U_pos) {
-            unsigned used = 0;
-            bool any = false;
-            for (int p = 0; p < g.U_pos; p++) {
-                if (done[p]) continue;
-                if (balanced && (mask_of[p] & used)) continue;
-                if (!balanced && any) break;
-                g.pos_order[n_out++] = (unsigned char)p; done[p] = true; used |= mask_of[p]; any = true;
-                if (mask_of[p] == 0) continue;                // (a position no pixel uses: cannot happen for full tiles)
-            }
-            if (!any) break;
-        }
-        for (int p = n_out; p < kMaxPos; p++) g.pos_order[p] = 0;
-    }
     KN_REQUIRE((size_t)(2 * n_slots + 2 * g.n_a + 2 * n_raw + 2) * 8 <= 1024, "spmm_tile_tc: too many barriers");
     g.n_slots = n_slots;
     g.n_raw = n_raw;
-    static const int bulk = getenv("KN_TILE_BULK") ? atoi(getenv("KN_TILE_BULK")) : 1;
     g.epi_pixels = (int)(((int64_t)n_raw * kRawStageBytes) / ((int64_t)G * BM * 4));
     if (g.epi_pixels > g.T) g.epi_pixels = g.T;
-    g.bulk_epi = (bulk && g.epi_pixels >= 1 && (((uintptr_t)Y) & 15) == 0 && ldy % 4 == 0) ? 1 : 0;
+    g.bulk_epi = (g.epi_pixels >= 1 && (((uintptr_t)Y) & 15) == 0 && ldy % 4 == 0) ? 1 : 0;
     const size_t smem = (size_t)n_slots * g.slab_bytes + (size_t)n_raw * kRawStageBytes + fixed;
     const int64_t n_btiles = kn_cdiv(n_vecs, BM);
     KN_REQUIRE(n_tiles * n_btiles <= 0x7fffffffLL, "spmm_tile_tc: grid too large");
     TileJobs jobs;
     memset(&jobs, 0, sizeof(jobs));
     for (int w = 0; w < g.n_iss; w++) {
-        for (int o = 0; o < g.U_pos; o++) {
-            const int p = g.pos_order[o];
+        for (int p = 0; p < g.U_pos; p++) {
             const int py = p / g.uw, px = p - py * g.uw;
             int tap0 = -1, m = 0, acc0 = 0, rel = 0;
             if (g.merged) {
@@ -644,7 +550,7 @@ KN_API int kn_spmm_tile_tc_f32(const void *maps_host, const int32_t *tile_cols, 
                 if (dy >= 0 && dy < g.P && dx >= 0 && dx < g.Q) { tap0 = dy * g.Q + dx; m = 1; acc0 = w; rel = 1; }
             }
             if (tap0 < 0) continue;
-            int4 &rec = jobs.rec[w * kMaxPos + o];
+            int4 &rec = jobs.rec[w * kMaxPos + p];
             rec.x = 2 | (rel << 2) | (tap0 << 8) | ((acc0 * g.Gp) << 16);
             rec.y = (int)(((1u << m) - 1u) << tap0);
             rec.z = (int)(((uint32_t)tap0 * (uint32_t)g.plane_bytes) >> 4);          // slab ring of exactly n_taps slots: slot = tap
@@ -655,23 +561,21 @@ KN_API int kn_spmm_tile_tc_f32(const void *maps_host, const int32_t *tile_cols, 
     memcpy(maps, maps_host, 4 * sizeof(CUtensorMap));
     const KnPeers peers = kn_current_peers();
     const bool relu = (flags & KN_SPMM_RELU) != 0;
-    const int super_ = tile_super_tiles();
     const dim3 grid((unsigned)(n_tiles * n_btiles));
     cudaStream_t s = (cudaStream_t)stream;
     // geometry-specialised issuers (issuer_fast) for 3x3 / stride-1 layers with the tile shapes the host picks
     const bool spec_ok = g.merged && g.ksplit == 2 && P == 3 && Q == 3 && stride == 1 && g.n_slots == 9;
     const int spec = !spec_ok ? 0 : (th == 2 && tw == 2 && g.Gp == 64) ? 1 : (th == 2 && tw == 2 && g.Gp == 96) ? 2 : (th == 1 && tw == 2 && g.Gp == 128) ? 3 : 0;
-#define KN_TILE_LAUNCH2(R, PP, A, B, C) do { \
-        auto kfn = pg_tile_tc_kernel<R, PP, A, B, C>; \
-        KN_ONCE_PER_DEVICE { KN_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); } \
-        kfn<<<grid, kThreads, smem, s>>>(maps[0], maps[1], tile_cols, tile_rows, bias_col, g, jobs, n_tiles, n_btiles, super_, X, ldx, Y, ldy, n_vecs, peers); } while (0)
-#define KN_TILE_LAUNCH(R, PP) do { \
-        if (spec == 1) KN_TILE_LAUNCH2(R, PP, 2, 2, 64); else if (spec == 2) KN_TILE_LAUNCH2(R, PP, 2, 2, 96); \
-        else if (spec == 3) KN_TILE_LAUNCH2(R, PP, 1, 2, 128); else KN_TILE_LAUNCH2(R, PP, 0, 0, 0); } while (0)
-    if (peers.n > 0) { if (relu) KN_TILE_LAUNCH(true, true); else KN_TILE_LAUNCH(false, true); }
-    else             { if (relu) KN_TILE_LAUNCH(true, false); else KN_TILE_LAUNCH(false, false); }
-#undef KN_TILE_LAUNCH
-#undef KN_TILE_LAUNCH2
-    KN_CHECK_LAUNCH();
-    return KN_OK;
+    return dispatch_relu_peers(relu, peers.n > 0, [&](auto R, auto PP) {
+        constexpr bool r = decltype(R)::value, pp = decltype(PP)::value;
+        const decltype(&pg_tile_tc_kernel<r, pp, 0, 0, 0>) kfns[4] = {pg_tile_tc_kernel<r, pp, 0, 0, 0>, pg_tile_tc_kernel<r, pp, 2, 2, 64>,
+                                                                      pg_tile_tc_kernel<r, pp, 2, 2, 96>, pg_tile_tc_kernel<r, pp, 1, 2, 128>};
+        KN_ONCE_PER_DEVICE {
+            for (auto kfn : kfns) KN_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        }
+        kfns[spec]<<<grid, kThreads, smem, s>>>(maps[0], maps[1], tile_cols, tile_rows, bias_col, g, jobs, n_tiles, n_btiles, kSuperTiles,
+                                                X, ldx, Y, ldy, n_vecs, peers);
+        KN_CHECK_LAUNCH();
+        return KN_OK;
+    });
 }

@@ -1,10 +1,22 @@
-// tc_common.cuh -- PTX wrappers shared by the tcgen05 kernels (pgroup_tc.cu, pgtile_tc.cu): mbarriers, TMA loads, UMMA
-// descriptors, tcgen05.mma / .st / .commit.  sm_100a only.
+// tc_common.cuh -- what the tcgen05 kernels (pgroup_tc.cu, pgtile_tc.cu) share: their stage / tile constants, PTX wrappers
+// (mbarriers, TMA loads, UMMA descriptors, tcgen05.mma / .ld / .st / .commit, TMEM allocation), the per-lane output store and
+// the launch dispatch.  sm_100a only.
 #pragma once
 #include "common.cuh"
 #include <cuda.h>
+#include <type_traits>
 
 namespace kn_tc {
+
+constexpr int KS = 16;                 // k per stage, = the TMA box width (words) of the weight planes (kn_pg_tc_tensormaps)
+constexpr int BM = 128;                // batch columns per UMMA (M): one per TMEM lane
+// rasterisation super-tile (kn_raster): 8 x 128 = 1024 batch columns, small enough that the X rows shared by neighbouring
+// groups (3x3 windows re-read every row 9 times, one image row of groups apart) are still L2-resident when they are re-read
+// (sweep 4..32: 4/8 best by ~1 %)
+constexpr int kSuperTiles = 8;
+// weight rows per UMMA (N) and per TMA box: G rounded up to the UMMA's N granularity of 16, at most 256 (a taller group
+// runs in 256-row chunks)
+__host__ __device__ constexpr int tc_gp(int G) { return G > 256 ? 256 : (G + 15) / 16 * 16; }
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -143,6 +155,75 @@ __device__ __forceinline__ void tmem_store(uint32_t taddr, const uint32_t (&r)[N
         asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
                      :: "r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]) : "memory");
     }
+}
+// 16 consecutive columns of the warp's 32 TMEM lanes (lane i of the warp gets TMEM lane (taddr >> 16) + i), waited for
+__device__ __forceinline__ void tmem_load16(uint32_t taddr, uint32_t (&r)[16]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
+                   "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                 : "r"(taddr));
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+}
+
+// All 512 TMEM columns for the CTA (the kernels run one CTA per SM); one whole warp calls both.  The base address lands in
+// *slot (shared memory) and is read after the next __syncthreads, between tc_fence_before / tc_fence_after.
+__device__ __forceinline__ void tmem_alloc512(uint32_t *slot) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" :: "r"(smem_u32(slot)));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+}
+// after tc_fence_before + __syncthreads: no tcgen05 operation of the CTA is outstanding
+__device__ __forceinline__ void tmem_dealloc512(uint32_t base) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" :: "r"(base));
+}
+
+// Per-lane epilogue of 16 accumulator columns of batch column ne (< n_vecs): r[t] (fp32 bits, ReLU applied here) goes to row
+// row_of(t) of Y for t < n_rows; the other columns have no row (row_of is not called for them).  PEERS (fused all-gather): to
+// that row of every destination whose bit is set in the row's need mask -- row ids and masks are loaded first (a load placed
+// between the stores would be serialised behind them), then one pass of stores per destination.  PEERS is a template
+// parameter because its code costs the plain epilogue ~10 %.  The plain path keeps each row-id load under the same guard as
+// its store: loading all 16 first made the compiler branch around every store instead of predicating it (pg_tc's conv
+// layers 1-2 % slower on a B200).
+template <bool RELU, bool PEERS, typename RowOf>
+__device__ __forceinline__ void store_rows16(uint32_t (&r)[16], int n_rows, RowOf row_of, float *__restrict__ Y, int64_t ldy, int64_t ne,
+                                             const KnPeers &peers) {
+    if constexpr (!PEERS) {
+#pragma unroll
+        for (int t = 0; t < 16; t++) {
+            if (t < n_rows) {
+                float y = __uint_as_float(r[t]);
+                if (RELU) y = fmaxf(y, 0.0f);
+                Y[(int64_t)row_of(t) * ldy + ne] = y;
+            }
+        }
+    } else {
+        int32_t yrow[16];
+        unsigned pmask[16];
+#pragma unroll
+        for (int t = 0; t < 16; t++) yrow[t] = (t < n_rows) ? row_of(t) : -1;
+#pragma unroll
+        for (int t = 0; t < 16; t++) pmask[t] = (yrow[t] >= 0) ? kn_peer_mask(peers, yrow[t]) : 0u;
+#pragma unroll
+        for (int t = 0; t < 16; t++) {
+            float y = __uint_as_float(r[t]);
+            if (RELU) y = fmaxf(y, 0.0f);
+            r[t] = __float_as_uint(y);
+        }
+        for (int p = 0; p < peers.n; p++) {
+            float *__restrict__ yb = peers.y[p];
+#pragma unroll
+            for (int t = 0; t < 16; t++)
+                if ((pmask[t] >> p) & 1u) yb[(int64_t)yrow[t] * ldy + ne] = __uint_as_float(r[t]);
+        }
+    }
+}
+
+// Host: calls launch(std::bool_constant<RELU>, std::bool_constant<PEERS>) for the run-time pair and returns its result, so a
+// kernel's launch code names its instantiation once.
+template <typename F>
+int dispatch_relu_peers(bool relu, bool peers, F &&launch) {
+    if (peers) return relu ? launch(std::true_type{}, std::true_type{}) : launch(std::false_type{}, std::true_type{});
+    return relu ? launch(std::true_type{}, std::false_type{}) : launch(std::false_type{}, std::false_type{});
 }
 
 

@@ -1076,15 +1076,9 @@ class PatternGroups(object):
     def _finish_class(cls, K_max, cid, n_cols):
         """Execution extras of one class: TF32 hi/lo planes + TMA descriptors for the tensor-core kernel, K slices for a
         single tall group (dense fc layers), the clustered form for short reductions (cid: cluster id per group, sorted)."""
-        L = _native.lib()
         (G, K_pad, ng, vals) = (cls['G'], cls['K_pad'], cls['n_groups'], cls['vals'])
         if G >= PatternGroups.TC_MIN_G and PatternGroups.TC_MIN_K <= K_pad <= PatternGroups.TC_MAX_K and tensor_cores_enabled():
-            # tensor-core operands: TF32 hi / bf16 corr planes of the value blocks + TMA descriptors (csrc/pgroup_tc.cu)
-            (vhi, vcorr) = (torch.empty_like(vals), torch.empty_like(vals))
-            check(L.kn_pg_tc_split(ptr(vals), vals.numel(), ptr(vhi), ptr(vcorr), stream_ptr()))
-            maps = ctypes.create_string_buffer(4 * 128)
-            check(L.kn_pg_tc_tensormaps(ptr(vhi), ptr(vcorr), cls['n_blocks'] * G, G, K_pad, maps))
-            cls['tc'] = dict(hi=vhi, corr=vcorr, maps=maps)
+            cls['tc'] = _tc_planes(vals, cls['n_blocks'] * G, G, K_pad)
         if cls['tc'] is not None and ng == 1 and K_max >= PatternGroups.SPLITK_MIN_K:
             cls['splitk'] = PatternGroups._split_k(cls, int(K_max))
         if cid is not None and K_pad <= PatternGroups.CG_KERNEL_MAX_K:
@@ -1098,7 +1092,6 @@ class PatternGroups(object):
     def _split_k(cls, K):
         """A class that is ONE group (all rows of a dense layer share the column set): S groups over K slices writing partial
         rows, so that row chunks x S >= the SM count.  Returns the inner class dict (own TF32 planes and TMA descriptors)."""
-        L = _native.lib()
         (G, K_pad) = (cls['G'], cls['K_pad'])
         dev = cls['vals'].device
         chunks = -(-G // 256) if G > 256 else 1                        # row chunks of the tensor-core kernel
@@ -1111,12 +1104,8 @@ class PatternGroups(object):
         cols_s = torch.cat([cols, cols[-1:].expand(pad)]).reshape(S, Kp).to(torch.int32).contiguous()
         vals_s = torch.cat([vals, torch.zeros((G, pad), dtype=torch.float32, device=dev)], dim=1).reshape(G, S, Kp).permute(1, 0, 2).contiguous().reshape(-1)
         group_k = torch.tensor([min(Kp, K - s * Kp) for s in range(S)], dtype=torch.int32, device=dev)
-        (vhi, vcorr) = (torch.empty_like(vals_s), torch.empty_like(vals_s))
-        check(L.kn_pg_tc_split(ptr(vals_s), vals_s.numel(), ptr(vhi), ptr(vcorr), stream_ptr()))
-        maps = ctypes.create_string_buffer(4 * 128)
-        check(L.kn_pg_tc_tensormaps(ptr(vhi), ptr(vcorr), S * G, G, Kp, maps))
         return dict(S=S, G=G, K_pad=Kp, rows=torch.arange(S * G, dtype=torch.int32, device=dev), cols=cols_s.reshape(-1), group_k=group_k,
-                    tc=dict(hi=vhi, corr=vcorr, maps=maps), part={})
+                    tc=_tc_planes(vals_s, S * G, G, Kp), part={})
 
     CG_MAX_G = 128           # groups up to this height are ordered by their spatial hint (L1 / L2 locality of the gathers)
     CG_KERNEL_MAX_K = 32     # ... and run on the clustered kernel when the reduction is short (K_pad <= 32: first conv layers,
@@ -1496,6 +1485,17 @@ def _keyed_conv_direct(geom, wq, bq, A, Ainv, rows, col_remap, n_cols_phys, want
 
 
 
+def _tc_planes(vals, n_rows, G, K_pad):
+    """Operands of the tensor-core kernels (csrc/pgroup_tc.cu, csrc/pgtile_tc.cu) for row-major value rows [n_rows][K_pad]
+    read in boxes of G rows: the TF32 hi / bf16 corr planes and their TMA descriptors (4 x 128 bytes, host memory)."""
+    L = _native.lib()
+    (hi, corr) = (torch.empty_like(vals), torch.empty_like(vals))
+    check(L.kn_pg_tc_split(ptr(vals), vals.numel(), ptr(hi), ptr(corr), stream_ptr()))
+    maps = ctypes.create_string_buffer(4 * 128)
+    check(L.kn_pg_tc_tensormaps(ptr(hi), ptr(corr), n_rows, G, K_pad, maps))
+    return dict(hi=hi, corr=corr, maps=maps)
+
+
 def _conv_tiles(desc, geom, wq, bq, pix_np, row_of_src, col_map, bias_col, dev):
     """Tile format of a conv layer for the spatially tiled tensor-core kernel (csrc/pgtile_tc.cu), or None when the layer
     does not qualify: G <= 128 output channels (taller groups are tensor-bound on the per-pixel kernel already), C a
@@ -1525,15 +1525,11 @@ def _conv_tiles(desc, geom, wq, bq, pix_np, row_of_src, col_map, bias_col, dev):
     Wt[:, :n_taps * C] = np.ascontiguousarray(wq, dtype=np.float32).reshape(M, C, n_taps).transpose(0, 2, 1).reshape(M, n_taps * C)      # k = tap * C + c
     Wt[:, n_taps * C] = bq
     w = torch.from_numpy(Wt).to(dev).reshape(-1)
-    (hi, corr) = (torch.empty_like(w), torch.empty_like(w))
-    check(L.kn_pg_tc_split(ptr(w), w.numel(), ptr(hi), ptr(corr), stream_ptr()))
-    maps = ctypes.create_string_buffer(4 * 128)
-    check(L.kn_pg_tc_tensormaps(ptr(hi), ptr(corr), M, M, K_pad, maps))
     t_origin = torch.from_numpy(tiles.astype(np.int32)).to(dev)
     tile_cols = torch.empty(n_tiles * uh * uw * C, dtype=torch.int32, device=dev)
     tile_rows = torch.empty(n_tiles * th * tw * M, dtype=torch.int32, device=dev)
     check(L.kn_conv2d_tiles_index(desc, ptr(t_origin), n_tiles, th, tw, ptr(row_of_src), ptr(col_map), ptr(tile_cols), ptr(tile_rows), stream_ptr()))
-    return dict(maps=maps, hi=hi, corr=corr, cols=tile_cols, rows=tile_rows, bias_col=bias_col, n_tiles=n_tiles, C=C, G=M, th=th, tw=tw, stride=stride, P=P, Q=Q)
+    return dict(_tc_planes(w, M, M, K_pad), cols=tile_cols, rows=tile_rows, bias_col=bias_col, n_tiles=n_tiles, C=C, G=M, th=th, tw=tw, stride=stride, P=P, Q=Q)
 
 
 def _recipe(kind, geom, A, Ainv, rows, col_remap, **extra):
