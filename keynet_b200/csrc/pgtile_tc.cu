@@ -281,14 +281,18 @@ pg_tile_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_const
         const float *__restrict__ xcol = X + (col_ok ? ncol : 0);
         const int bytes = col_ok ? 16 : 0;                      // src-size 0 => 16 bytes of zeros
         const int mine = warp - kGatherWarp0;
+        // A warp waits for its slot by parity only, which is sound while the slot's previous lap has been consumed: with g
+        // warps taking turns, a warp's previous stage waited for the consumption of stage i - g - n_raw, so g <= n_raw
+        // gather warps at most (a 6-stage ring under 7 warps overwrote unconsumed stages and hung: G = 128, C = 512).
+        const int n_gw = geo.n_raw < kGatherWarps ? geo.n_raw : kGatherWarps;
         int i = -1, cc = 0, p = -1;                              // stage counter and its (chunk, union position)
-        int slot = -1, turn = kGatherWarps - 1; uint32_t rph = 1u;   // the stage's ring slot / the parity its raw_empty is waited with / whose turn it is
-        while (true) {
+        int slot = -1, turn = n_gw - 1; uint32_t rph = 1u;       // the stage's ring slot / the parity its raw_empty is waited with / whose turn it is
+        while (mine < n_gw) {
             // next in-image stage, chunk-major; after the last chunk the bias stage (ring position kept incrementally: a runtime
             // division per stage is ~150 cycles of a gather warp's ~460)
             ++i;
             if (++slot == geo.n_raw) { slot = 0; rph ^= 1u; }
-            if (++turn == kGatherWarps) turn = 0;
+            if (++turn == n_gw) turn = 0;
             if (i == n_stages - 1) p = kBiasPos;
             else if (i >= n_stages) break;
             else do { if (++p == U_pos) { p = 0; ++cc; } } while (!((vmask >> p) & 1u));
