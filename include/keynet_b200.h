@@ -128,6 +128,21 @@ int kn_spmm_pg_f32(const int32_t *rows, const int32_t *cols, const float *vals, 
  * Y[rows[i]][:] = relu?(sum_s part[s*G + i][:]) (and performs the peer stores of the row-sharded path). */
 int kn_splitk_reduce_f32(const float *part, int32_t S, int32_t G, const int32_t *rows, float *Y, int64_t ldy, int64_t n_vecs, uint32_t flags, const kn_peers *peers, void *stream);
 
+/* Narrow batches (csrc/pgroup.cu): same contract as kn_spmm_pg_f32 for 1 <= n_vecs <= 32, with any ldx / ldy >= n_vecs and
+ * any 4-byte alignment of X and Y (no padding of the batch to 32 columns).
+ *   run_groups[n_groups], run_start[n_runs+1]  run table: the class's groups listed run by run; a run is at most
+ *                            128 / NB groups (NB = n_vecs rounded up to a power of two) that share one value block
+ *                            (block_of) and one group_k.  Required whenever n_groups > 0.
+ *   row_form = 0             shared-block form (pg_simt over runs): the tile's 128 columns are (group, batch column) pairs
+ *                            of one run, the run's value rows are staged once and serve all its groups; per output element
+ *                            the same fp32 FMA chain as kn_spmm_pg_f32's pg_simt kernel (bit-identical results).
+ *   row_form = 1             row form (n_vecs <= 8; CSR kernel spmm_lanes_nnz over the class's rows): one warp per row,
+ *                            lanes over the group's first group_k columns, fixed shuffle reduction (deterministic).
+ * peers must be NULL: the fused row-sharded path pads its batch to the grouped kernels itself. */
+int kn_spmm_pg_narrow_f32(const int32_t *rows, const int32_t *cols, const float *vals, const int32_t *group_k, const int32_t *block_of, int64_t n_groups, int32_t G, int32_t K_pad,
+                          const int32_t *run_groups, const int32_t *run_start, int64_t n_runs, int32_t row_form,
+                          const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, uint32_t flags, const kn_peers *peers, void *stream);
+
 /* Clustered variant for short reductions (csrc/pgcluster.cu; G <= 256, walked 16 rows at a time above 16): the groups of a tile of neighbouring output pixels
  * form a cluster with ONE union column list that is staged in shared memory once per (cluster, 128 batch columns), so a
  * 3x3 convolution reads every X row from L2 about once instead of 9 times.

@@ -24,6 +24,7 @@ SYMBOLS = [
     'kn_conv2d_tiles_index', 'kn_spmm_tile_tc_f32', 'kn_convpool_f32',
     'kn_keyed_conv2d_count', 'kn_keyed_conv2d_fill', 'kn_conv2d_groups_index', 'kn_conv2d_groups_values',
     'kn_spgemm_bound', 'kn_spgemm_rows', 'kn_csr_compact', 'kn_encrypt_monomial_t', 'kn_splitk_reduce_f32',
+    'kn_spmm_pg_narrow_f32',
 ]
 
 
@@ -91,6 +92,7 @@ def lib():
         'kn_pg_verify': [vp, vp, vp, vp, i64, vp, vp],
         'kn_pg_pack': [vp, vp, vp, vp, i64, ctypes.c_int32, ctypes.c_int32, vp, vp, vp],
         'kn_spmm_pg_f32': [vp, vp, vp, vp, vp, i64, ctypes.c_int32, ctypes.c_int32, vp, i64, vp, i64, i64, u32, pp, vp],
+        'kn_spmm_pg_narrow_f32': [vp, vp, vp, vp, vp, i64, ctypes.c_int32, ctypes.c_int32, vp, vp, i64, ctypes.c_int32, vp, i64, vp, i64, i64, u32, pp, vp],
         'kn_spmm_cg_f32': [vp, vp, vp, vp, vp, vp, vp, vp, i64, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, vp, i64, vp, i64, i64, u32, pp, vp],
         'kn_debug_tc_timing': [ctypes.c_int32, vp],
         'kn_encrypt_monomial_t': [vp, i64, i64, vp, vp, vp, vp, i64, vp],

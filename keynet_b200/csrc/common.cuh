@@ -74,6 +74,17 @@ struct KnPeersScope {
     ~KnPeersScope();
 };
 
+// Rows of one pattern-group class (csrc/pgroup.cu) as the CSR kernel's row source: row i of the product is row i % G of
+// group i / G, its entries the group's first group_k[g] columns cols[g][k] with values vals[block_of[g]][i % G][k], written to
+// Y[rows[i]].  The row form of narrow batches (kn_spmm_pg_narrow_f32): one warp per row, lanes over the row's columns.
+struct KnGroupRows {
+    const int32_t *rows = nullptr, *cols = nullptr, *group_k = nullptr, *block_of = nullptr;
+    const float *vals = nullptr;
+    int G = 0, K_pad = 0;
+};
+// n_rows = n_groups * G rows, 1 <= n_vecs <= 8 (csrc/spmm.cu); plain stores, no peers
+int kn_spmm_group_rows(const KnGroupRows &gr, int64_t n_rows, const float *X, int64_t ldx, float *Y, int64_t ldy, int n_vecs, bool relu, cudaStream_t s);
+
 // number of SMs of the current device (cached); B200 = 148
 int kn_sm_count();
 

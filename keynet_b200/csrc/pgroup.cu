@@ -96,14 +96,28 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src,
     const int bytes = valid ? 16 : 0;                     // src-size 0 => 16 bytes of zeros
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" :: "r"(dst), "l"(gmem_src), "r"(bytes));
 }
+__device__ __forceinline__ void cp_async4(void *smem_dst, const void *gmem_src, bool valid) {
+    const unsigned dst = (unsigned)__cvta_generic_to_shared(smem_dst);
+    const int bytes = valid ? 4 : 0;                      // src-size 0 => 4 bytes of zeros
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;\n" :: "r"(dst), "l"(gmem_src), "r"(bytes));
+}
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" :: "n"(N)); }
+
+// Narrow batches (1 <= n_vecs <= 32, run_start != null; kn_spmm_pg_narrow_f32): a 128-column tile would hold n_vecs useful
+// columns, so its columns become (group, batch column) pairs, j = p * NB + n with NB = 1 << nb_shift >= n_vecs.  A work item
+// is then a RUN -- run_groups[run_start[i] .. run_start[i+1]), at most 128 / NB groups sharing one value block and one
+// group_k -- so the staged value rows serve every group of the run.  The B stage gathers X[cols[g_p][k]][n] with 4-byte
+// cp.async (zero for n >= n_vecs and for missing groups: any ldx and alignment); the FMA loop is the same as for wide
+// batches, so every output element is the same fp32 chain (bit-identical to a wide launch over a zero-padded X).
+constexpr int kNarrowMaxRW = 4;   // narrow batches use row tiles of 8, 16 or 32 rows: a thin grid needs CTAs more than long tiles
 
 template <int RW, bool RELU>
 __global__ void __launch_bounds__(kThreads, 2)
 pg_simt_kernel(const int32_t *__restrict__ rows, const int32_t *__restrict__ cols, const float *__restrict__ vals,
                const int32_t *__restrict__ group_k, const int32_t *__restrict__ block_of, int64_t n_groups, int G, int K_pad, int tiles_per_group, int64_t n_items, int64_t n_tiles,
-               const float *__restrict__ X, int64_t ldx, float *__restrict__ Y, int64_t ldy, int64_t n_vecs, const __grid_constant__ KnPeers peers)
+               const float *__restrict__ X, int64_t ldx, float *__restrict__ Y, int64_t ldy, int64_t n_vecs, const __grid_constant__ KnPeers peers,
+               const int32_t *__restrict__ run_groups, const int32_t *__restrict__ run_start, int nb_shift)
 {
     constexpr int TM = 8 * RW;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -112,9 +126,13 @@ pg_simt_kernel(const int32_t *__restrict__ rows, const int32_t *__restrict__ col
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const KnRaster rt = kn_raster(blockIdx.x, n_items, n_tiles, 16);      // super-tile = 16 x 128 batch columns
-    const int64_t g = rt.item / tiles_per_group;
-    const int rowtile = (int)(rt.item - g * tiles_per_group);
+    const int64_t item = rt.item / tiles_per_group;                       // group, or run of groups (narrow)
+    const int rowtile = (int)(rt.item - item * tiles_per_group);
     const int64_t nbase = rt.tile * TN;
+    const bool narrow = RW <= kNarrowMaxRW && run_start != nullptr;    // compiled out of the taller row tiles
+    const int r0 = narrow ? __ldg(run_start + item) : 0;
+    const int n_here = narrow ? __ldg(run_start + item + 1) - r0 : 1;   // groups of the run (<= 128 >> nb_shift)
+    const int64_t g = narrow ? (int64_t)__ldg(run_groups + r0) : item;
     // groups of one class share K_pad (storage) but loop only over their own K (edge / corner pixels have fewer taps)
     const int n_chunks = group_k ? (__ldg(group_k + g) + KT - 1) / KT : K_pad / KT;
 
@@ -122,6 +140,11 @@ pg_simt_kernel(const int32_t *__restrict__ rows, const int32_t *__restrict__ col
     const float *__restrict__ vbase = vals + (blk * G + (int64_t)rowtile * TM) * K_pad;
     const int32_t *__restrict__ cbase = cols + g * (int64_t)K_pad;
     const int rows_here = min(TM, G - rowtile * TM);
+    // narrow: this thread's B-stage column (group p of the run, batch column n), fixed over the k loop
+    const int jb = tid & (TN - 1), pb = jb >> nb_shift, nb = jb & ((1 << nb_shift) - 1);
+    const bool jok = narrow && pb < n_here && nb < n_vecs;
+    const int32_t *__restrict__ cb = narrow ? cols + (int64_t)__ldg(run_groups + r0 + (jok ? pb : 0)) * K_pad : cbase;
+    const float *__restrict__ xb = X + (jok ? nb : 0);
 
     auto load_stage = [&](int s, int kc) {
         // A: TM rows x 8 chunks of 16 B
@@ -133,6 +156,15 @@ pg_simt_kernel(const int32_t *__restrict__ rows, const int32_t *__restrict__ col
                 const bool ok = r < rows_here;
                 cp_async16(&sA[s][r][ch * 4], vbase + (ok ? ((int64_t)r * K_pad + kc * KT + ch * 4) : 0), ok);
             }
+        }
+        if (narrow) {
+            // B: per thread one tile column, 16 of the 32 gathered rows, 4 bytes each
+#pragma unroll
+            for (int i = 0; i < (KT * TN) / kThreads; i++) {
+                const int kr = (tid >> 7) + i * (kThreads / TN);
+                cp_async4(&sB[s][kr][jb], xb + (int64_t)__ldg(cb + kc * KT + kr) * ldx, jok);
+            }
+            return;
         }
         // B: 32 gathered X rows x 32 chunks of 16 B (one warp per row: 512 contiguous bytes)
 #pragma unroll
@@ -182,6 +214,21 @@ pg_simt_kernel(const int32_t *__restrict__ rows, const int32_t *__restrict__ col
     }
     cp_async_wait<0>();
 
+    if (narrow) {                                                    // scalar stores of the (group, column) pairs
+#pragma unroll
+        for (int c = 0; c < 4; c++) {
+            const int j = lane * 4 + c, p = j >> nb_shift, n = j & ((1 << nb_shift) - 1);
+            if (p < n_here && n < n_vecs) {
+                const int64_t rbase = (int64_t)__ldg(run_groups + r0 + p) * G + (int64_t)rowtile * TM;
+#pragma unroll
+                for (int i = 0; i < RW; i++) {
+                    const int r = warp * RW + i;
+                    if (r < rows_here) Y[(int64_t)__ldg(rows + rbase + r) * ldy + n] = RELU ? fmaxf(acc[i][c], 0.0f) : acc[i][c];
+                }
+            }
+        }
+        return;
+    }
     const int64_t n0 = nbase + lane * 4;
     if (n0 < n_vecs) {
 #pragma unroll
@@ -343,22 +390,26 @@ int launch_small(const int32_t *rows, const int32_t *cols, const float *vals, co
     return KN_OK;
 }
 
+// run_start != null: narrow batches over the n_runs runs of the run table, NB = 1 << nb_shift (see pg_simt_kernel)
 template <int RW>
 int launch_pg(const int32_t *rows, const int32_t *cols, const float *vals, const int32_t *group_k, const int32_t *block_of, int64_t n_groups, int G, int K_pad,
-              const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, bool relu, cudaStream_t s)
+              const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, bool relu, cudaStream_t s,
+              const int32_t *run_groups = nullptr, const int32_t *run_start = nullptr, int64_t n_runs = 0, int nb_shift = 0)
 {
     constexpr int TM = 8 * RW;
     const size_t smem = sizeof(float) * kStages * (TM * KT + KT * TN);
     const int tiles_per_group = (G + TM - 1) / TM;
-    const int64_t gx = n_groups * tiles_per_group, gy = kn_cdiv(n_vecs, TN);
+    const int64_t gx = (run_start ? n_runs : n_groups) * tiles_per_group, gy = run_start ? 1 : kn_cdiv(n_vecs, TN);
     KN_REQUIRE(gx * gy <= 0x7fffffffLL, "spmm_pg: grid too large");
     KN_ONCE_PER_DEVICE {
         KN_CUDA(cudaFuncSetAttribute(pg_simt_kernel<RW, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         KN_CUDA(cudaFuncSetAttribute(pg_simt_kernel<RW, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
     dim3 grid((unsigned)(gx * gy));
-    if (relu) pg_simt_kernel<RW, true><<<grid, kThreads, smem, s>>>(rows, cols, vals, group_k, block_of, n_groups, G, K_pad, tiles_per_group, gx, gy, X, ldx, Y, ldy, n_vecs, kn_current_peers());
-    else      pg_simt_kernel<RW, false><<<grid, kThreads, smem, s>>>(rows, cols, vals, group_k, block_of, n_groups, G, K_pad, tiles_per_group, gx, gy, X, ldx, Y, ldy, n_vecs, kn_current_peers());
+    if (relu) pg_simt_kernel<RW, true><<<grid, kThreads, smem, s>>>(rows, cols, vals, group_k, block_of, n_groups, G, K_pad, tiles_per_group, gx, gy, X, ldx, Y, ldy, n_vecs, kn_current_peers(),
+                                                                    run_groups, run_start, nb_shift);
+    else      pg_simt_kernel<RW, false><<<grid, kThreads, smem, s>>>(rows, cols, vals, group_k, block_of, n_groups, G, K_pad, tiles_per_group, gx, gy, X, ldx, Y, ldy, n_vecs, kn_current_peers(),
+                                                                     run_groups, run_start, nb_shift);
     KN_CHECK_LAUNCH();
     return KN_OK;
 }
@@ -437,4 +488,31 @@ KN_API int kn_spmm_pg_f32(const int32_t *rows, const int32_t *cols, const float 
     const int waste96 = ((G + 95) / 96) * 96 - G, waste128 = ((G + 127) / 128) * 128 - G;
     if (waste96 < waste128) return launch_pg<12>(rows, cols, vals, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s);
     return launch_pg<16>(rows, cols, vals, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s);
+}
+
+KN_API int kn_spmm_pg_narrow_f32(const int32_t *rows, const int32_t *cols, const float *vals, const int32_t *group_k, const int32_t *block_of, int64_t n_groups, int32_t G, int32_t K_pad,
+                                 const int32_t *run_groups, const int32_t *run_start, int64_t n_runs, int32_t row_form,
+                                 const float *X, int64_t ldx, float *Y, int64_t ldy, int64_t n_vecs, uint32_t flags, const kn_peers *peers, void *stream) {
+    KN_REQUIRE(peers == nullptr, "spmm_pg_narrow: no output peers (the fused row-sharded path pads its batch to the grouped kernels)");
+    KN_REQUIRE(n_vecs >= 1 && n_vecs <= 32, "spmm_pg_narrow: n_vecs must be in 1..32 (got %lld)", (long long)n_vecs);
+    KN_REQUIRE(ldx >= n_vecs && ldy >= n_vecs, "spmm_pg_narrow: bad leading dimension");
+    KN_REQUIRE(n_groups >= 0 && G > 0 && K_pad > 0 && K_pad % KT == 0, "spmm_pg_narrow: bad shape (G=%d K_pad=%d)", G, K_pad);
+    KN_REQUIRE(row_form == 0 || (row_form == 1 && n_vecs <= 8), "spmm_pg_narrow: the row form (row_form = 1) serves n_vecs <= 8 (row_form=%d)", row_form);
+    if (n_groups == 0) return KN_OK;
+    KN_REQUIRE(run_groups && run_start && n_runs > 0 && n_runs <= n_groups, "spmm_pg_narrow: empty run table (%lld runs for %lld groups)", (long long)n_runs, (long long)n_groups);
+    KN_REQUIRE(rows && cols && vals && X && Y, "spmm_pg_narrow: null pointer");
+    KnPeersScope peers_scope(nullptr);
+    cudaStream_t s = (cudaStream_t)stream;
+    const bool relu = (flags & KN_SPMM_RELU) != 0;
+    if (row_form) {
+        KnGroupRows gr;
+        (gr.rows = rows, gr.cols = cols, gr.group_k = group_k, gr.block_of = block_of, gr.vals = vals, gr.G = G, gr.K_pad = K_pad);
+        return kn_spmm_group_rows(gr, n_groups * G, X, ldx, Y, ldy, (int)n_vecs, relu, s);
+    }
+    int nb_shift = 0;
+    while ((1 << nb_shift) < n_vecs) nb_shift++;
+    static_assert(kNarrowMaxRW == 4, "the dispatch below stops at pg_simt<4>");
+    if (G <= 8)  return launch_pg<1>(rows, cols, vals, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s, run_groups, run_start, n_runs, nb_shift);
+    if (G <= 16) return launch_pg<2>(rows, cols, vals, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s, run_groups, run_start, n_runs, nb_shift);
+    return launch_pg<4>(rows, cols, vals, group_k, block_of, n_groups, G, K_pad, X, ldx, Y, ldy, n_vecs, relu, s, run_groups, run_start, n_runs, nb_shift);
 }

@@ -14,7 +14,8 @@
 //     moment work on the SAME batch chunk: that chunk's slab of X (C x 128V bytes) is what has
 //     to live in L2, not all of X.
 //   * lanes_nnz<NB> (N <= 8): one warp per row, lanes stride over the row's entries (coalesced
-//     index/value reads), NB accumulators per lane, warp-shuffle tree reduction at the end.
+//     index/value reads), NB accumulators per lane, warp-shuffle tree reduction at the end.  It also takes its rows from a
+//     pattern-group class (KnGroupRows, common.cuh): the row form of narrow batches on layers without a CSR.
 #include "common.cuh"
 #include <stdlib.h>
 
@@ -192,13 +193,22 @@ __global__ void __launch_bounds__(kWarps * 32)
 spmm_lanes_nnz_kernel(const int64_t *__restrict__ indptr, const int32_t *__restrict__ indices,
                       const float *__restrict__ data, int64_t n_rows,
                       const float *__restrict__ X, int64_t ldx, float *__restrict__ Y, int64_t ldy, int n_vecs,
-                      const int32_t *__restrict__ out_rows, const __grid_constant__ KnPeers peers)
+                      const int32_t *__restrict__ out_rows, const __grid_constant__ KnPeers peers, const KnGroupRows gr)
 {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t row = (int64_t)blockIdx.x * kWarps + warp;
     if (row >= n_rows) return;
-    const int64_t beg = indptr[row], end = indptr[row + 1];
-    const int64_t yrow = out_rows ? (int64_t)out_rows[row] : row;
+    int64_t beg, end, yrow;
+    if (gr.cols == nullptr) {
+        beg = indptr[row]; end = indptr[row + 1];
+        yrow = out_rows ? (int64_t)out_rows[row] : row;
+    } else {                                       // row row % G of pattern group row / G: its entries start at offset 0
+        const int64_t g = row / gr.G, blk = gr.block_of ? (int64_t)__ldg(gr.block_of + g) : g;
+        indices = gr.cols + g * gr.K_pad;
+        data = gr.vals + (blk * gr.G + (row - g * gr.G)) * gr.K_pad;
+        beg = 0; end = gr.group_k ? __ldg(gr.group_k + g) : gr.K_pad;
+        yrow = __ldg(gr.rows + row);
+    }
     const unsigned pmask = kn_peer_mask(peers, yrow);
     float acc[NB];
 #pragma unroll
@@ -252,17 +262,26 @@ int launch_rowwarp_wide(const int64_t *indptr, const int32_t *indices, const flo
 
 template <int NB>
 int launch_lanes(const int64_t *indptr, const int32_t *indices, const float *data, int64_t n_rows,
-                 const float *X, int64_t ldx, float *Y, int64_t ldy, int n_vecs, bool relu, const int32_t *out_rows, cudaStream_t s)
+                 const float *X, int64_t ldx, float *Y, int64_t ldy, int n_vecs, bool relu, const int32_t *out_rows, cudaStream_t s,
+                 const KnGroupRows &gr = KnGroupRows())
 {
     const int64_t gx = kn_cdiv(n_rows, kWarps);
     KN_REQUIRE(gx <= 0x7fffffffLL, "spmm: too many rows (%lld)", (long long)n_rows);
-    if (relu) spmm_lanes_nnz_kernel<NB, true><<<(unsigned)gx, kWarps * 32, 0, s>>>(indptr, indices, data, n_rows, X, ldx, Y, ldy, n_vecs, out_rows, kn_current_peers());
-    else      spmm_lanes_nnz_kernel<NB, false><<<(unsigned)gx, kWarps * 32, 0, s>>>(indptr, indices, data, n_rows, X, ldx, Y, ldy, n_vecs, out_rows, kn_current_peers());
+    if (relu) spmm_lanes_nnz_kernel<NB, true><<<(unsigned)gx, kWarps * 32, 0, s>>>(indptr, indices, data, n_rows, X, ldx, Y, ldy, n_vecs, out_rows, kn_current_peers(), gr);
+    else      spmm_lanes_nnz_kernel<NB, false><<<(unsigned)gx, kWarps * 32, 0, s>>>(indptr, indices, data, n_rows, X, ldx, Y, ldy, n_vecs, out_rows, kn_current_peers(), gr);
     KN_CHECK_LAUNCH();
     return KN_OK;
 }
 
 }  // namespace
+
+int kn_spmm_group_rows(const KnGroupRows &gr, int64_t n_rows, const float *X, int64_t ldx, float *Y, int64_t ldy, int n_vecs, bool relu, cudaStream_t s)
+{
+    if (n_vecs == 1) return launch_lanes<1>(nullptr, nullptr, nullptr, n_rows, X, ldx, Y, ldy, n_vecs, relu, nullptr, s, gr);
+    if (n_vecs == 2) return launch_lanes<2>(nullptr, nullptr, nullptr, n_rows, X, ldx, Y, ldy, n_vecs, relu, nullptr, s, gr);
+    if (n_vecs <= 4) return launch_lanes<4>(nullptr, nullptr, nullptr, n_rows, X, ldx, Y, ldy, n_vecs, relu, nullptr, s, gr);
+    return launch_lanes<8>(nullptr, nullptr, nullptr, n_rows, X, ldx, Y, ldy, n_vecs, relu, nullptr, s, gr);
+}
 
 static int spmm_csr_impl(const int64_t *indptr, const int32_t *indices, const float *data,
                          int64_t n_rows, int64_t n_cols, const int32_t *out_rows,

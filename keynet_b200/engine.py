@@ -94,7 +94,13 @@ class ForwardPlan(object):
                 else:
                     i += 1
         skip = set(i + 1 for i in self.fused)
-        self.launches_per_run = (1 if self.fused_encrypt else 3) + sum(0 if i in skip else (1 if i in self.fused else (W._pg.launches() if (W._pg is not None and N >= 32 and N % 4 == 0) else 1))
+        def spmm_launches(W):
+            if W._pg is not None and N >= 32 and N % 4 == 0:
+                return W._pg.launches()
+            if W._pg is not None and W._data is None and N < 32:
+                return W._pg.launches_narrow()
+            return 1
+        self.launches_per_run = (1 if self.fused_encrypt else 3) + sum(0 if i in skip else (1 if i in self.fused else spmm_launches(W))
                                                                         for (i, (_, W, _)) in enumerate(self.layers) if i >= 1)
         self.time_layers = time_layers
         # per-layer CUDA events on the launch stream, one set per timed step (read back after the timed region)

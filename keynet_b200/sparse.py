@@ -1179,6 +1179,62 @@ class PatternGroups(object):
             check(L.kn_spmm_csr_rows_f32(ptr(r['indptr']), ptr(r['indices']), ptr(r['data']), r['n'], self.shape[1], ptr(r['out_rows']),
                                          ptr(x), N, ptr(y), N, N, flags, pp, stream_ptr()))
 
+    NARROW_TILE = 128        # batch-column slots of pg_simt's tile: a run of the narrow path holds up to 128 / NB groups
+
+    @staticmethod
+    def _run_table(cls, P):
+        """The class's groups ordered by (value block, group_k) and cut into runs of at most P groups that share both:
+        dict(groups int32 [n_groups] run by run, start int32 [n_runs + 1], n_runs)."""
+        ng = cls['n_groups']
+        dev = cls['cols'].device
+        blk = cls['block_of'].to(torch.int64) if cls['block_of'] is not None else torch.arange(ng, dtype=torch.int64, device=dev)
+        key = blk * (cls['K_pad'] + 1) + cls['group_k'].to(torch.int64)
+        (ks, order) = torch.sort(key, stable=True)
+        new = torch.ones(ng, dtype=torch.bool, device=dev)
+        new[1:] = ks[1:] != ks[:-1]
+        seg_start = torch.nonzero(new).reshape(-1)
+        pos = torch.arange(ng, device=dev) - seg_start[torch.cumsum(new.to(torch.int64), 0) - 1]     # position inside its block
+        start = torch.nonzero(pos % P == 0).reshape(-1)
+        start = torch.cat([start, torch.tensor([ng], device=dev)]).to(torch.int32).contiguous()
+        return dict(groups=order.to(torch.int32).contiguous(), start=start, n_runs=int(start.numel()) - 1)
+
+    @staticmethod
+    def _narrow_plan(cls, N):
+        """How the class runs at 1 <= N < 32 batch columns (cached per NB on the class: built by the first call, so a CUDA
+        graph captured after a warm-up run allocates nothing).  Row form (row_form = 1: one warp per row, lanes over K) when
+        NB <= 8 and the shared-block tile would be less than a quarter full (mean run length x NB < 32 of its 128 columns);
+        shared-block form otherwise.  Dense fc layers (one group) and gain-keyed layers (a block per group) take the row form
+        up to N = 8; convolutions under permutation keys take the shared form except where few pixels share a block (VGG16
+        conv5 at N = 1: 196 pixels, ~20 per run)."""
+        NB = 1 << max(0, (int(N) - 1).bit_length())
+        plans = cls.setdefault('narrow', {})
+        p = plans.get(NB)
+        if p is None:
+            p = PatternGroups._run_table(cls, PatternGroups.NARROW_TILE // NB)
+            p.update(NB=NB, row_form=int(NB <= 8 and cls['n_groups'] * NB < 32 * p['n_runs']))
+            plans[NB] = p
+        return p
+
+    def spmm_narrow(self, x, y, relu):
+        """Y = W . X for 1 <= N < 32 batch columns, no output peers (kn_spmm_pg_narrow_f32): no padding of the batch."""
+        L = _native.lib()
+        N = x.shape[1]
+        assert 1 <= N < 32
+        flags = _native.KN_SPMM_RELU if relu else 0
+        for c in self.classes:
+            p = PatternGroups._narrow_plan(c, N)
+            check(L.kn_spmm_pg_narrow_f32(ptr(c['rows']), ptr(c['cols']), ptr(c['vals']), ptr(c['group_k']), ptr(c['block_of']), c['n_groups'], c['G'], c['K_pad'],
+                                          ptr(p['groups']), ptr(p['start']), p['n_runs'], p['row_form'],
+                                          ptr(x), N, ptr(y), N, N, flags, None, stream_ptr()))
+        r = self.rest
+        if r is not None:
+            check(L.kn_spmm_csr_rows_f32(ptr(r['indptr']), ptr(r['indices']), ptr(r['data']), r['n'], self.shape[1], ptr(r['out_rows']),
+                                         ptr(x), N, ptr(y), N, N, flags, None, stream_ptr()))
+
+    def launches_narrow(self):
+        """Kernel launches of spmm_narrow: one per class and one for `rest`."""
+        return len(self.classes) + (1 if self.rest is not None else 0)
+
     def launches(self):
         return sum(2 if c.get('splitk') is not None else 1 for c in self.classes) + (1 if self.rest is not None else 0)
 
@@ -1202,11 +1258,14 @@ def spmm(W, x, relu=False, out=None, peers=None):
         W._pg.spmm(x, y, relu, peers)
         return y
     if W._data is None:
-        # CSR was dropped (drop_csr): narrow / ragged batches are padded to the grouped kernels' granularity
-        Np = max(32, (N + 3) // 4 * 4)
         # the grouped kernels would store into the peers' buffers with leading dimension Np: the fused row-sharded path
         # must pad its batch itself (dist.ShardedKeyedModel does)
         assert peers is None, 'ragged batch on a dropped-CSR matrix with output peers: the fused row-sharded path pads its batch itself'
+        if 0 < N < 32:
+            W._pg.spmm_narrow(x, y, relu)
+            return y
+        # CSR was dropped (drop_csr): ragged batches are padded to the grouped kernels' granularity
+        Np = max(32, (N + 3) // 4 * 4)
         xp = torch.zeros((x.shape[0], Np), dtype=torch.float32, device=x.device)
         xp[:, :N] = x
         yp = torch.empty((R, Np), dtype=torch.float32, device=x.device)
